@@ -208,6 +208,31 @@ def parity_check(wl, dens, seed, queries, rows, threads):
             "score_compare": "bit-equal", "oracle_s": round(time.perf_counter() - t0, 2)}
 
 
+DUMP_LIMIT_BYTES = 64_000_000 - 4096  # 64 MB in all, the five .npy headers included
+
+
+def dump_outputs(path, rows, seed):
+    """Writes one step's result rows so that two builds can be compared output for output: scores.npy (float32 [n, k]),
+    segment_ords.npy, docs.npy (float64 [n, k], exact for u32), counts.npy and queries.npy (float64 [n]: the rows' positions in
+    the batch).  Entries past a query's count are zero.  When the batch's rows exceed DUMP_LIMIT_BYTES, n is a sample of the
+    queries drawn from `seed`, the same for every run with the same arguments."""
+    scores, segs, docs, counts = (np.asarray(a) for a in rows)
+    nq, k = scores.shape
+    row_bytes = k * (4 + 8 + 8) + 8 + 8
+    queries = np.arange(nq)
+    if nq * row_bytes > DUMP_LIMIT_BYTES:
+        queries = np.sort(np.random.default_rng(seed).choice(nq, DUMP_LIMIT_BYTES // row_bytes, replace=False))
+    valid = np.arange(k)[None, :] < np.minimum(counts[queries], k)[:, None]
+    os.makedirs(path, exist_ok=True)
+    out = {"scores": np.where(valid, scores[queries], 0).astype(np.float32),
+           "segment_ords": np.where(valid, segs[queries], 0).astype(np.float64),
+           "docs": np.where(valid, docs[queries], 0).astype(np.float64),
+           "counts": counts[queries].astype(np.float64),
+           "queries": queries.astype(np.float64)}
+    for name, a in out.items():
+        np.save(os.path.join(path, name + ".npy"), a)
+
+
 def cpu_reference_run(wl, shard, batches, steps, warmup, sample_queries, threads):
     """The reference CPU algorithm (oracle restatement, Block-WAND + TopNHeap + merge_top_k), all host
     cores, on a bounded sample of the same query stream. One step = `sample_queries` queries."""
@@ -246,7 +271,14 @@ def main():
                     help="batches in flight per GPU in the timed legs (2: step i+1 is queued on its own stream before the host waits for step i; "
                          "0 = auto: 2 on one GPU, 1 at N > 1, where queueing step i+1 early skews the ranks between the key exchanges of step i "
                          "and measured 4 %% slower at N = 2)")
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the rows the last timed step returned (scores, segment ords, docs, counts) as DIR/<name>.npy, "
+                         "float32 / float64, at most 64 MB (a seeded sample of the queries beyond that)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        ap.error("--dump-outputs writes the product arm's rows; the reference arm times a sample of the query stream")
     if args.warmup < 3:
         args.warmup = 3
 
@@ -397,6 +429,13 @@ def main():
     dt_value = time.perf_counter() - t0
     touched_per_step = (stats["or_windows"][5] - touched0) / max(args.steps, 1) if stats else 0
     clocks = sampler.stop() if sampler else None
+    if args.dump_outputs and rank == 0:  # the rows of the last timed step, read back after the timed region
+        if world > 1:
+            m = mergers[(args.steps - 1) % depth]
+            last_rows = m._host_views(m.rows_o.cpu().numpy())
+        else:
+            last_rows = prepared[(args.warmup + args.steps - 1) % n_prep].fetch()
+        dump_outputs(args.dump_outputs, last_rows, args.seed)
     for b in prepared:
         b.close()
 
