@@ -152,13 +152,12 @@ typedef struct {
   float term_ms, and_ms, or_ms, final_ms; /* per-kernel device time (CUDA events on the launching stream) */
   uint64_t units_term, units_and, units_or; /* CTAs launched per kernel */
   uint64_t bytes_term, bytes_and, bytes_or; /* algorithmic bytes per kernel (same formula) */
-  /* cumulative since ctx creation.  k_or_strip (default union kernel): [1] windows scored exhaustively (no
-   * non-essential clause under the threshold), [2] hot windows (non-essential clauses applied after the essential
-   * ones), [3] cold windows (essential clauses only), [5] bytes of packed postings + fieldnorms actually read
-   * (SURVEY.md §8d: the roofline figure of a pruned kernel).  k_or with TQ_OR_PRUNE=1 uses the slots for its own
-   * routes (0 skipped, 1 exhaustive, 2 MaxScore route, 3 no promising doc, 4/5 overflows, 6/7 docs/postings scored). */
+  /* cumulative since ctx creation, written by k_or_strip only: [1] windows scored exhaustively (no non-essential
+   * clause under the threshold), [2] hot windows (non-essential clauses applied after the essential ones), [3] cold
+   * windows (essential clauses only), [5] bytes of packed postings + fieldnorms actually read (SURVEY.md §8d: the
+   * roofline figure of a pruned kernel).  [0], [4], [6] and [7] are always 0. */
   uint64_t or_windows[8];
-  uint64_t units_or_strip; /* of units_or: CTAs of the barrier-free strip kernel (k_or_strip); the rest ran k_or / k_or_pipe */
+  uint64_t units_or_strip; /* of units_or: CTAs of the barrier-free strip kernel (k_or_strip); the rest ran k_or */
   /* shared-decode tile engine (k_score_lists + k_tile, csrc/tq_tile.cuh) */
   float score_ms, tile_ms, theta_ms;  /* device time of k_score_lists / all k_tile launches / the k_theta passes of the batch */
   float phrase_ms;                    /* device time of k_phrase */

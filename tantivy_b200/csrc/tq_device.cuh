@@ -101,13 +101,11 @@ struct BatchParams {
   uint32_t* res_counts;
   uint32_t res_stride;
   uint32_t n_queries;
-  unsigned long long* counters;  // [8] k_or window routes: 0 skipped, 1 exhaustive, 2 pruned+scored, 3 pruned+empty,
-                                 //     4 essential overflow, 5 promising overflow, 6 promising docs, 7 essential postings
-  uint32_t or_prune;             // 0 disables the MaxScore route of k_or (A/B measurements)
-  uint32_t strip_prune;          // 0 disables the essential / non-essential split of k_or_strip
-  uint32_t strip_ne_div;         // clauses with >= 1 posting per this many docs may turn non-essential
-  uint32_t strip_ne_div2;        // ...and the densest clause of a union without such a clause, under this looser bound
-  uint32_t* ovf;                 // set by k_final when a query was handed more candidates than its region holds (tile engine only), or null
+  unsigned long long* counters;  // [8] k_or_strip diagnostics, tq_stats.or_windows
+  // Unused.  Every kernel takes BatchParams by value; with 16 bytes less, ptxas schedules k_tile's parameter loads
+  // differently and the default workload measured 0.2 % slower (B200, 1000 W power limit).
+  uint32_t reserved[4];
+  uint32_t* ovf;                // set by k_final when a query was handed more candidates than its region holds (tile engine only), or null
 };
 
 // ---- small helpers ---------------------------------------------------------------------------
@@ -302,13 +300,8 @@ struct TopK {
   unsigned int* count;        // shared
   unsigned long long* theta;  // shared: keys below it can no longer enter the top-k
   TopKScratch* scratch;       // shared
-  unsigned long long* counters;  // global diagnostics (BatchParams::counters)
-  unsigned named;     // 0: the whole CTA takes part (__syncthreads); 1: only the first `nthreads` threads (bar.sync 1)
-  unsigned nthreads;  // threads that take part (threadIdx.x < nthreads)
+  unsigned nthreads;          // threads of the CTA
 };
-__device__ __forceinline__ void topk_sync(const TopK& t) {
-  if (t.named) asm volatile("bar.sync 1, 256;" ::: "memory"); else __syncthreads();
-}
 
 // All lanes of a warp call this together (pass may differ per lane).
 __device__ __forceinline__ void topk_push(const TopK& t, bool pass, unsigned long long key, uint32_t lane) {
@@ -323,13 +316,13 @@ __device__ __forceinline__ void topk_push(const TopK& t, bool pass, unsigned lon
 
 // Whole CTA. Sorts the buffer (descending) and keeps the best k; publishes the k-th score.
 __device__ __noinline__ void topk_compact(const TopK& t, uint32_t k, unsigned int* theta_global) {
-  topk_sync(t);
+  __syncthreads();
   const unsigned n = *t.count;
   unsigned size = 2;
   while (size < n) size <<= 1;
   for (unsigned i = threadIdx.x; i < size; i += t.nthreads)
     if (i >= n) t.keys[i] = 0ull;
-  topk_sync(t);
+  __syncthreads();
   for (unsigned kk = 2; kk <= size; kk <<= 1) {
     for (unsigned j = kk >> 1; j > 0; j >>= 1) {
       for (unsigned i = threadIdx.x; i < size; i += t.nthreads) {
@@ -340,7 +333,7 @@ __device__ __noinline__ void topk_compact(const TopK& t, uint32_t k, unsigned in
           if (desc ? (a < b) : (a > b)) { t.keys[i] = b; t.keys[ixj] = a; }
         }
       }
-      topk_sync(t);
+      __syncthreads();
     }
   }
   if (threadIdx.x == 0 && n > k) {
@@ -349,7 +342,7 @@ __device__ __noinline__ void topk_compact(const TopK& t, uint32_t k, unsigned in
     if (kth > *t.theta) *t.theta = kth;
     atomicMax(theta_global, (unsigned)(kth >> 32));
   }
-  topk_sync(t);
+  __syncthreads();
 }
 
 // Cheap compaction.  The CTA only has to keep a SUPERSET of its k best keys and a threshold that is a valid
@@ -359,12 +352,12 @@ __device__ __noinline__ void topk_compact(const TopK& t, uint32_t k, unsigned in
 // part.  Falls back to the exact sort when the boundary bin is too crowded (ties) to make room.
 __device__ __noinline__ void topk_compact_hist(const TopK& t, uint32_t k, uint32_t keep_max, unsigned int* theta_global) {
   TopKScratch& sc = *t.scratch;
-  topk_sync(t);
+  __syncthreads();
   const unsigned n = *t.count;
   if (n <= k) return;  // uniform
   for (unsigned i = threadIdx.x; i < 256; i += t.nthreads) sc.hist[i] = 0;
   if (threadIdx.x == 0) { sc.kmin = 0xFFFFFFFFu; sc.kmax = 0; sc.hole_n = 0; sc.mover_n = 0; }
-  topk_sync(t);
+  __syncthreads();
   unsigned lmin = 0xFFFFFFFFu, lmax = 0;
   for (unsigned i = threadIdx.x; i < n; i += t.nthreads) {
     const unsigned sk = (unsigned)(t.keys[i] >> 32);
@@ -373,11 +366,11 @@ __device__ __noinline__ void topk_compact_hist(const TopK& t, uint32_t k, uint32
   lmin = __reduce_min_sync(kFull, lmin);
   lmax = __reduce_max_sync(kFull, lmax);
   if ((threadIdx.x & 31u) == 0) { atomicMin(&sc.kmin, lmin); atomicMax(&sc.kmax, lmax); }
-  topk_sync(t);
+  __syncthreads();
   const unsigned kmin = sc.kmin, span = sc.kmax - kmin;
   const unsigned shift = span < 256u ? 0u : (unsigned)(32 - __clz(span)) - 8u;  // (key - kmin) >> shift in [0, 255]
   for (unsigned i = threadIdx.x; i < n; i += t.nthreads) atomicAdd(&sc.hist[((unsigned)(t.keys[i] >> 32) - kmin) >> shift], 1u);
-  topk_sync(t);
+  __syncthreads();
   if (threadIdx.x < 32) {  // suffix sums over the 256 bins: 8 per lane
     const unsigned lane = threadIdx.x;
     unsigned loc[8], tot = 0;
@@ -404,9 +397,8 @@ __device__ __noinline__ void topk_compact_hist(const TopK& t, uint32_t k, uint32
     keep = __shfl_sync(kFull, keep, src);
     if (lane == 0) { sc.cut = (unsigned)cut; sc.keep = keep; }
   }
-  topk_sync(t);
+  __syncthreads();
   const unsigned keep = sc.keep;
-  if (threadIdx.x == 0) { atomicAdd(&t.counters[3], 1ull); if (keep > keep_max || keep == n) atomicAdd(&t.counters[4], 1ull); }
   if (keep > keep_max || keep == n) {  // crowded boundary bin (ties) or nothing to drop: exact route
     topk_compact(t, k, theta_global);
     return;
@@ -414,41 +406,41 @@ __device__ __noinline__ void topk_compact_hist(const TopK& t, uint32_t k, uint32
   const unsigned edge = kmin + (sc.cut << shift);  // every survivor has score key >= edge, and there are >= k of them
   for (unsigned i = threadIdx.x; i < keep; i += t.nthreads)
     if ((unsigned)(t.keys[i] >> 32) < edge) sc.holes[atomicAdd(&sc.hole_n, 1u)] = (unsigned short)i;
-  topk_sync(t);
+  __syncthreads();
   for (unsigned i = keep + threadIdx.x; i < n; i += t.nthreads) {
     const unsigned long long key = t.keys[i];
     if ((unsigned)(key >> 32) >= edge) t.keys[sc.holes[atomicAdd(&sc.mover_n, 1u)]] = key;
   }
-  topk_sync(t);
+  __syncthreads();
   if (threadIdx.x == 0) {
     *t.count = keep;
     const unsigned long long th = (unsigned long long)edge << 32;
     if (th > *t.theta) *t.theta = th;
     atomicMax(theta_global, edge);
   }
-  topk_sync(t);
+  __syncthreads();
 }
 
 // End of a round of the CTA: refresh the shared threshold from the query-wide one and make room.
 // `limit`: compact as soon as this many keys are buffered (a pruning kernel wants its threshold early).
 __device__ __forceinline__ void topk_round_end(const TopK& t, uint32_t k, unsigned int* theta_global, uint32_t limit = kCap - kRoundMargin) {
-  topk_sync(t);
+  __syncthreads();
   if (*t.count > limit) topk_compact_hist(t, k, kCap - kRoundMargin, theta_global);
   if (threadIdx.x == 0) {
     const unsigned long long g = (unsigned long long)(*(volatile unsigned int*)theta_global) << 32;
     if (g > *t.theta) *t.theta = g;
   }
-  topk_sync(t);
+  __syncthreads();
 }
 
 // End of a unit: the CTA's survivors go to the query's candidate region (at most 2k of them).
 __device__ __noinline__ void topk_flush(const TopK& t, const DQuery& q, QState* qs, Cand* cands, uint32_t segment_ord) {
-  topk_sync(t);
+  __syncthreads();
   if (*t.count > 2u * q.k) topk_compact_hist(t, q.k, min(2u * q.k, kCap / 2u), &qs->theta);
   __shared__ unsigned s_base;
   const unsigned n = *t.count;
   if (threadIdx.x == 0) s_base = n ? atomicAdd(&qs->cand_count, n) : 0u;
-  topk_sync(t);
+  __syncthreads();
   const unsigned base = s_base;
   for (unsigned i = threadIdx.x; i < n; i += t.nthreads) {
     if (base + i < q.cand_cap) {

@@ -140,8 +140,8 @@ struct tq_ctx {
   DevBuf build_dev;
   std::vector<tq_batch*> pool;
   tq_stats stats{};
-  uint32_t term_blocks_per_unit, and_blocks_per_unit, or_tiles_per_unit;
-  unsigned long long* d_counters = nullptr;  // [0..8) k_or / k_or_strip window routes, [8..16) k_tile diagnostics
+  uint32_t term_blocks_per_unit, and_blocks_per_unit;
+  unsigned long long* d_counters = nullptr;  // [0..8) k_or_strip diagnostics (or_windows), [8..16) k_tile diagnostics
   uint32_t tile = 1, tile_scratch_mb = 24576, tile_sample_div = 16, tile_round_div1 = 8, tile_round_div2 = 2, tile_light_max = 96, tile_counters = 0;
   uint32_t tile_ops = 7;  // bit per TQ_OP_*: which query shapes the tile engine takes
   uint32_t tile_seg_cap_hook = 0;
@@ -151,7 +151,6 @@ struct tq_ctx {
   uint32_t tile_max_slots = kTileMaxSlots, tile_max_queries = kTileMaxQueries, tile_wide_queries = 256;
   uint64_t tile_smem_last = 0;
   uint32_t tile_cand_floor = 32768, tile_max_dens_x1000 = 0, tile_pcap_hook = 0, tile_big_min = 6, tile_units = 148 * 6;
-  uint32_t or_prune = 1, or_strip = 1, or_pipe = 1, strip_prune = 1, strip_sample_div = 32, strip_sample_div2 = 8, strip_sample_div3 = 2, strip_ne_div = 8, strip_ne_div2 = 64;
 };
 
 constexpr int kTileRounds = 4;  // launches of k_tile per run: the sample launch + three exact ones
@@ -200,7 +199,6 @@ struct tq_batch {
   uint32_t phrase_ct = 2;                 // most terms of a phrase in the batch (k_phrase's candidate stride)
   const PhraseAux* phrase_aux = nullptr;  // device: per clause of the batch's phrase queries (parallel to qlists)
   uint32_t strip_cached_max = 0;
-  uint32_t or_max_lists = 0;  // most clauses of any window-kernel union in the batch
   size_t qinit_off = 0;
   int next_phase = 0;  // of the current run (0: none started)
   size_t qstate_off = 0, cands_off = 0, res_off = 0, res_bytes = 0, n_cands = 0;
@@ -243,16 +241,6 @@ int tq_ctx_create(int device, tq_ctx** out) {
   c->lists_cap = env_u32("TQ_MAX_LISTS", 1u << 20);
   c->term_blocks_per_unit = env_u32("TQ_TERM_BLOCKS_PER_UNIT", 512);
   c->and_blocks_per_unit = env_u32("TQ_AND_BLOCKS_PER_UNIT", 128);
-  c->or_tiles_per_unit = env_u32("TQ_OR_TILES_PER_UNIT", 16);
-  c->or_strip = env_u32("TQ_OR_STRIP", 1);
-  c->or_pipe = env_u32("TQ_OR_PIPE", 1);
-  c->strip_sample_div = env_u32("TQ_STRIP_SAMPLE_DIV", 32);  // share of a pair's windows in the threshold sample (0/1: off)
-  c->strip_sample_div2 = env_u32("TQ_STRIP_SAMPLE_DIV2", 8);  // second sample round ends at this share (0/1: one round only)
-  c->strip_sample_div3 = env_u32("TQ_STRIP_SAMPLE_DIV3", 2);  // third round: up to half of the windows
-  c->strip_ne_div = env_u32("TQ_STRIP_NE_DIV", 8);
-  c->strip_ne_div2 = env_u32("TQ_STRIP_NE_DIV2", 64);
-  c->strip_prune = env_u32("TQ_STRIP_PRUNE", 1);  // MaxScore split inside k_or_strip (exact)
-  c->or_prune = env_u32("TQ_OR_PRUNE", 0);  // MaxScore route: exact, but only pays off for small k / rare terms
   c->tile = env_u32("TQ_TILE", 1);                          // unions take the shared-decode tile engine (tq_tile.cuh); 0 = per-query kernels only
   c->tile_scratch_mb = env_u32("TQ_TILE_SCRATCH_MB", 24576);  // (doc, score) pairs one batch may materialise
   c->tile_sample_div = env_u32("TQ_TILE_SAMPLE_DIV", 16);    // share of the tiles in the sample launch (0/1: none)
@@ -283,7 +271,6 @@ int tq_ctx_create(int device, tq_ctx** out) {
   if (err == cudaSuccess) err = cudaMemset(c->d_counters, 0, 16 * sizeof(unsigned long long));
   if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&c->build_stream, cudaStreamNonBlocking);
   if (err == cudaSuccess) err = cudaFuncSetAttribute(k_or, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kOrDynSmem);
-  if (err == cudaSuccess) err = cudaFuncSetAttribute(k_or_pipe, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)pipe_smem_bytes());
   if (err == cudaSuccess) err = cudaFuncSetAttribute(k_or_strip, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)strip_smem_bytes(kMaxCached));
   if (err == cudaSuccess) err = cudaFuncSetAttribute(k_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   if (err != cudaSuccess) { delete c; return fail(TQ_ERR_CUDA, cudaGetErrorString(err)); }
@@ -945,7 +932,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   std::vector<uint32_t> qseg_total;
   uint32_t n_qsegs_op[4] = {0, 0, 0, 0};
   std::vector<char> qseg_sample;  // strip pairs that get a threshold sample pass (MaxScore can then skip their dense clauses)
-  uint32_t strip_cached_max = 0, or_max_lists = 0, phrase_ct = 2;
+  uint32_t strip_cached_max = 0, phrase_ct = 2;
   std::vector<TileGroupBuild> tgroups;
   std::vector<size_t> q_cands(nq, 0);
   const bool tile_on = c->tile != 0 && !force_legacy;
@@ -1124,11 +1111,10 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
           for (auto& h : here) { qaux.push_back(PhraseAux{h.second.pad, h.range_len, q.slop}); h.second.pad = 0; }
           phrase_ct = std::max<uint32_t>(phrase_ct, (uint32_t)here.size());
         }
-        if (op == TQ_OP_OR && c->or_strip && q.k <= kStripMaxK && here.size() <= kStripMaxLists) {
+        if (op == TQ_OP_OR && q.k <= kStripMaxK && here.size() <= kStripMaxLists) {
           // strip kernel: clauses with less than one block per kWin-doc window keep their current block decoded in shared memory
           uint32_t n_thin = 0;
-          static const uint64_t thin_mult = env_u32("TQ_STRIP_THIN_MULT", 1u);
-          auto is_thin = [&](uint32_t df) { return (uint64_t)df * (kWin / 128u) < (uint64_t)qs.max_doc * thin_mult; };
+          auto is_thin = [&](uint32_t df) { return (uint64_t)df * (kWin / 128u) < (uint64_t)qs.max_doc; };
           for (auto& h : here) if (is_thin(h.first)) ++n_thin;
           if (n_thin <= kMaxCached) {
             uint32_t slot = 0;
@@ -1137,7 +1123,6 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
             unit_class = 3;
           }
         }
-        if (unit_class == TQ_OP_OR) or_max_lists = std::max<uint32_t>(or_max_lists, (uint32_t)here.size());
         for (auto& h : here) qlists.push_back(h.second);
         qs.n_lists = (uint32_t)here.size();
         const uint32_t lead_total = here[0].first / 128u + ((here[0].first % 128u) ? 1u : 0u);
@@ -1145,7 +1130,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
         qseg_op.push_back(unit_class);
         {
           bool any_thick = false;
-          for (auto& h : here) any_thick = any_thick || (uint64_t)h.first * std::max(c->strip_ne_div, c->strip_ne_div2) >= qs.max_doc;
+          for (auto& h : here) any_thick = any_thick || (uint64_t)h.first * std::max(kStripNeDiv, kStripNeDiv2) >= qs.max_doc;
           qseg_sample.push_back(unit_class == 3 && prunable && any_thick);
         }
         qseg_total.push_back(unit_class == 3 ? (qs.max_doc + kWin - 1) / kWin : (op == TQ_OP_OR ? (qs.max_doc + kTileDocs - 1) / kTileDocs : lead_total));
@@ -1159,19 +1144,19 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
     for (size_t s = 0; s < qsegs.size(); ++s) {
       const int op = qseg_op[s];
       const uint32_t total = qseg_total[s];
-      const uint32_t min_per = op == TQ_OP_TERM ? c->term_blocks_per_unit : ((op == TQ_OP_AND || op == 7) ? c->and_blocks_per_unit : (op == 3 ? kStripWarps * 64u : c->or_tiles_per_unit));
+      const uint32_t min_per = op == TQ_OP_TERM ? c->term_blocks_per_unit : ((op == TQ_OP_AND || op == 7) ? c->and_blocks_per_unit : (op == 3 ? kStripWarps * 64u : 16u));
       const uint32_t n_same = n_qsegs_op[op == 7 ? TQ_OP_AND : op];
       const uint32_t want_units = std::max<uint32_t>(1u, (target_units + n_same - 1) / n_same);
       const uint32_t per = std::max<uint32_t>(min_per, (total + want_units - 1) / want_units);
       const uint32_t k = dq[qsegs[s].query].k;
-      // Threshold sample: the first 1/sample_div of a strip pair's windows run in a launch of their own; the exact k-th
-      // best score over all sampled windows of the query (k_theta) then seeds the threshold of the main launch, whose
-      // MaxScore split drops the dense clauses from the first window on.  Nothing is scored twice.
+      // Threshold rounds: the first 1/32, then up to 1/8 and up to 1/2 of a strip pair's windows run in launches of their
+      // own; the exact k-th best score over all windows run so far of the query (k_theta) then seeds the threshold of the
+      // next launch, whose MaxScore split drops the dense clauses from the first window on.  Nothing is scored twice.
       uint32_t first = 0;
-      if (op == 3 && qseg_sample[s] && c->strip_sample_div > 1 && total >= 8u * c->strip_sample_div) {
-        const uint32_t cut1 = std::max<uint32_t>(kStripWarps, total / c->strip_sample_div);
-        const uint32_t cut2 = c->strip_sample_div2 > 1 && c->strip_sample_div2 < c->strip_sample_div ? std::max(cut1, total / c->strip_sample_div2) : cut1;
-        const uint32_t cut3 = c->strip_sample_div3 > 1 && c->strip_sample_div3 < c->strip_sample_div2 ? std::max(cut2, total / c->strip_sample_div3) : cut2;
+      if (op == 3 && qseg_sample[s] && total >= 8u * 32u) {
+        const uint32_t cut1 = std::max<uint32_t>(kStripWarps, total / 32u);
+        const uint32_t cut2 = std::max(cut1, total / 8u);
+        const uint32_t cut3 = std::max(cut2, total / 2u);
         const uint32_t cuts[4] = {0, cut1, cut2, cut3};
         for (int r = 0; r < 3; ++r)  // round r covers [cuts[r], cuts[r+1]); a k_theta pass follows each round
           for (uint32_t b0 = cuts[r]; b0 < cuts[r + 1]; b0 += per) {
@@ -1331,7 +1316,6 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   const size_t o_qaux = off; off = align(off + qaux.size() * sizeof(PhraseAux));
   const size_t n_units_total = units[0].size() + units[1].size() + units[2].size() + units[3].size() + units[4].size() + units[5].size() + units[6].size() + units[7].size();
   b->strip_cached_max = strip_cached_max;
-  b->or_max_lists = or_max_lists;
   b->phrase_ct = std::min<uint32_t>(phrase_ct, kPhraseMaxTerms);
   const size_t o_units = off; off = align(off + n_units_total * sizeof(Unit));
   const size_t o_queries = off; off = align(off + dq.size() * sizeof(DQuery));
@@ -1531,10 +1515,6 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   P.res_stride = kmax;
   P.n_queries = (uint32_t)nq;
   P.counters = c->d_counters;
-  P.or_prune = c->or_prune;
-  P.strip_prune = c->strip_prune;
-  P.strip_ne_div = c->strip_ne_div;
-  P.strip_ne_div2 = c->strip_ne_div2;
   P.ovf = b->groups.empty() ? nullptr : reinterpret_cast<uint32_t*>(b->tile_dev.p + to_flags) + 1;
 
   TQ_CUDA(cudaEventRecord(b->ev_start, b->stream));
@@ -1625,12 +1605,7 @@ static int run_phase(tq_batch* b, int phase) {
     }
     if (b->n_units[TQ_OP_OR]) {
       const int sp = span_begin(b, SPAN_OR);
-      // window unions: the TMA/mbarrier pipeline when every union has few enough clauses for its tables, else the plain kernel
-      if (b->ctx->or_pipe && b->or_max_lists <= kPipeMaxLists && !b->ctx->or_prune)
-        k_or_pipe<<<b->n_units[TQ_OP_OR], kPipeThreads, pipe_smem_bytes(), b->stream>>>(P, b->unit_base[TQ_OP_OR]);
-      else
-        k_or<<<b->n_units[TQ_OP_OR], kThreads, kOrDynSmem, b->stream>>>(P, b->unit_base[TQ_OP_OR]);
-      ++launches;
+      k_or<<<b->n_units[TQ_OP_OR], kThreads, kOrDynSmem, b->stream>>>(P, b->unit_base[TQ_OP_OR]); ++launches;
       span_end(b, sp);
     }
     if (tiles) {  // K1 + K2 once for every distinct list of the batch

@@ -228,7 +228,7 @@ __global__ void __launch_bounds__(kThreads) k_term(const BatchParams P, uint32_t
   const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
   if (threadIdx.x == 0) { s_top.count = 0; s_top.theta = (unsigned long long)qs->theta << 32; }
   __syncthreads();
-  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, P.counters, 0u, (unsigned)kThreads};
+  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, (unsigned)kThreads};
   BlockFetch f;
   if (U.begin + warp < U.end) fetch_issue(L, U.begin + warp, lane, f);
   for (uint32_t r = U.begin; r < U.end; r += kWarps) {
@@ -276,7 +276,7 @@ __global__ void __launch_bounds__(kThreads) k_and(const BatchParams P, uint32_t 
   uint32_t* dec = s_dec[warp];
   if (threadIdx.x == 0) { s_top.count = 0; s_top.theta = (unsigned long long)qs->theta << 32; }
   __syncthreads();
-  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, P.counters, 0u, (unsigned)kThreads};
+  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, (unsigned)kThreads};
   // MaxScore for the conjunction (exact): a leader doc whose own score plus the secondaries' bounds (score < weight)
   // cannot reach the threshold is dropped BEFORE its secondary blocks are looked up and decoded -- the lookups are
   // what this kernel spends its time on (block_wand_intersection.rs:60-120 prunes on block maxima for the same reason).
@@ -371,30 +371,16 @@ __global__ void __launch_bounds__(kThreads) k_and(const BatchParams P, uint32_t 
 // A slot holding -0.0f has not been touched: -0.0 + s == 0.0 + s bit for bit for every s except
 // s == -0.0 (SumCombiner starts from 0.0, score_combiner.rs:39-57).
 //
-// Two ways through a window of kTileDocs doc ids:
-//  * exhaustive: every clause's blocks are decoded and added in clause order, then the window is harvested;
-//  * MaxScore-pruned (once the threshold is high enough): clauses whose maximum scores add up to less
-//    than the threshold are "non-essential" (find_pivot_doc's prefix, block_wand_union.rs:16-43). Only the
-//    essential clauses are decoded; a doc is "promising" if its essential score plus the non-essential
-//    bound can reach the threshold, and only promising docs get their exact clause-ordered score.
-//    Every doc that is skipped provably scores below the threshold, so the result set is unchanged.
-constexpr uint32_t kTouchedCap = 2048;
-constexpr uint32_t kPromisingCap = 64;
-
+// The general per-query union (any number of clauses, any k): per window of kTileDocs doc ids every clause's blocks
+// are decoded and added in clause order, then the window is harvested.  A window is skipped when no clause has a
+// block in it, or when the clause maxima together cannot reach the threshold.
 struct OrShared {
   uint32_t blo[2][32], bhi[2][32];  // per clause: block range overlapping the tile (double buffered)
   uint32_t cur[32];                 // per clause: search cursor
   uint32_t any[2];
   uint32_t npass;
-  float prefix[33];      // prefix[i] = sum of the i smallest clause maxima
-  uint8_t order[32];     // clause ordinals by ascending maximum score
-  uint32_t ne_mask;      // non-essential clauses for the current threshold
-  float ne_bound;        // upper bound of their joint contribution
-  uint32_t mode;         // 0 skip, 1 exhaustive, 2 pruned
-  uint32_t touched_n, p_n, overflow;
-  uint16_t touched[kTouchedCap];
-  uint16_t plist[kPromisingCap];
-  uint32_t pbits[kTileDocs / 32];
+  float bound;                      // no doc of the segment scores above this
+  uint32_t skip;                    // the current window holds nothing that can enter the top-k
 };
 
 __device__ __forceinline__ void or_tile_ranges(const BatchParams& P, const QSeg& S, OrShared& sh, int buf, uint32_t tile,
@@ -445,25 +431,24 @@ __global__ void __launch_bounds__(kThreads, 3) k_or(const BatchParams P, uint32_
   const float neg_zero = __uint_as_float(0x80000000u);
   const bool staged_fn = (S.flags & 1u) && S.fieldnorm != nullptr;
   for (uint32_t i = threadIdx.x; i < kTileDocs; i += kThreads) s_acc[i] = neg_zero;
-  for (uint32_t i = threadIdx.x; i < kTileDocs / 32; i += kThreads) sh.pbits[i] = 0;
   if (threadIdx.x < 32) sh.cur[threadIdx.x] = 0;
   if (threadIdx.x == 0) {
     s_top.count = 0; s_top.theta = (unsigned long long)qs->theta << 32;
-    sh.any[0] = sh.any[1] = 0; sh.npass = 0; sh.touched_n = 0; sh.p_n = 0; sh.overflow = 0;
-    // clauses by ascending maximum score; a clause can add at most its weight (tf/(tf+norm) < 1, bm25.rs:170-175)
+    sh.any[0] = sh.any[1] = 0; sh.npass = 0;
+    // a clause can add at most its weight (tf/(tf+norm) < 1, bm25.rs:170-175); the maxima are summed smallest first
     float mx[32];
-    for (uint32_t t = 0; t < S.n_lists; ++t) { mx[t] = fmaxf(P.qlists[S.lists_base + t].weight, 0.0f); sh.order[t] = (uint8_t)t; }
-    for (uint32_t i = 1; i < S.n_lists; ++i) {
-      const uint8_t o = sh.order[i];
-      uint32_t j = i;
-      while (j > 0 && mx[sh.order[j - 1]] > mx[o]) { sh.order[j] = sh.order[j - 1]; --j; }
-      sh.order[j] = o;
+    for (uint32_t t = 0; t < S.n_lists; ++t) {
+      const float m = fmaxf(P.qlists[S.lists_base + t].weight, 0.0f);
+      uint32_t j = t;
+      while (j > 0 && mx[j - 1] > m) { mx[j] = mx[j - 1]; --j; }
+      mx[j] = m;
     }
-    sh.prefix[0] = 0.0f;
-    for (uint32_t i = 0; i < S.n_lists; ++i) sh.prefix[i + 1] = sh.prefix[i] + mx[sh.order[i]];
+    float sum = 0.0f;
+    for (uint32_t t = 0; t < S.n_lists; ++t) sum += mx[t];
+    sh.bound = sum * 1.00001f;  // f32 sums of up to 32 terms differ by < 4e-6 relative
   }
   __syncthreads();
-  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, P.counters, 0u, (unsigned)kThreads};
+  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, (unsigned)kThreads};
   or_tile_ranges(P, S, sh, 0, U.begin, warp, lane);
   unsigned int theta_g_seen = 0;  // thread 0: query-wide threshold sampled one window ago
   __syncthreads();
@@ -471,152 +456,19 @@ __global__ void __launch_bounds__(kThreads, 3) k_or(const BatchParams P, uint32_
     const int buf = (int)((tile - U.begin) & 1u);
     const uint32_t lo = tile * kTileDocs;
     const uint32_t hi = min(lo + kTileDocs, S.max_doc);
-    // ---- decide how to go through this window ------------------------------------------------------
     if (threadIdx.x == 0) {
       const unsigned long long g = (unsigned long long)theta_g_seen << 32;
       if (g > s_top.theta) s_top.theta = g;
       theta_g_seen = *(volatile unsigned int*)&qs->theta;  // consumed at the next window
-      const float theta_f = threshold_score((uint32_t)(s_top.theta >> 32));
-      uint32_t n_ne = 0, mask = 0;
-      while (n_ne < S.n_lists && sh.prefix[n_ne + 1] * 1.00001f < theta_f) { mask |= 1u << sh.order[n_ne]; ++n_ne; }
-      sh.ne_mask = mask;
-      sh.ne_bound = sh.prefix[n_ne] * 1.00001f;  // f32 sums of up to 32 terms differ by < 4e-6 relative
-      if (!P.or_prune && n_ne != S.n_lists) { n_ne = 0; sh.ne_mask = 0; sh.ne_bound = 0.0f; }
-      sh.mode = (!sh.any[buf] || n_ne == S.n_lists) ? 0u : (n_ne == 0 ? 1u : 2u);  // all non-essential: nothing here can enter the top-k
-      atomicAdd(&P.counters[sh.mode == 0 ? 0 : (sh.mode == 1 ? 1 : 2)], 1ull);
+      sh.skip = !sh.any[buf] || sh.bound < threshold_score((uint32_t)(s_top.theta >> 32));
     }
     __syncthreads();
-    uint32_t mode = sh.mode;
+    const bool skip = sh.skip != 0;
     const unsigned long long theta = *T.theta;
     const float theta_f = threshold_score((uint32_t)(theta >> 32));
 
-    if (mode == 2) {
-      // ---- pruned, stage 1: essential clauses only, order-free estimate ---------------------------
-      const uint32_t ne_mask = sh.ne_mask;
-      uint32_t rr = 0;
-      for (uint32_t t = 0; t < S.n_lists; ++t) {
-        if ((ne_mask >> t) & 1u) continue;
-        const uint32_t blo = sh.blo[buf][t], bhi = sh.bhi[buf][t];
-        if (blo > bhi) continue;
-        const uint32_t nb = bhi - blo + 1u;
-        const QList ql = P.qlists[S.lists_base + t];
-        const ListDesc L = P.lists[ql.list_id];
-        const Scorer scr = make_scorer(P, ql);
-        for (uint32_t b = blo + ((warp + kWarps - (rr & (kWarps - 1))) & (kWarps - 1)); b <= bhi; b += kWarps) {
-          uint32_t doc[4], tf[4];
-          decode_block(L, b, lane, doc, tf);
-#pragma unroll
-          for (int i = 0; i < 4; ++i) {
-            if (doc[i] >= lo && doc[i] < hi) {
-              const uint32_t slot = doc[i] - lo;
-              const float sc = bm25_score(scr, L.fieldnorm, doc[i], tf[i]);
-              const float old = atomicAdd(&s_acc[slot], sc);
-              if (__float_as_uint(old) == 0x80000000u) {
-                const uint32_t idx = atomicAdd(&sh.touched_n, 1u);
-                if (idx < kTouchedCap) sh.touched[idx] = (uint16_t)slot; else sh.overflow = 1;
-              }
-            }
-          }
-        }
-        rr += nb;
-      }
-      __syncthreads();
-      if (sh.overflow) {  // too many essential postings for the list: clean up and take the exhaustive route
-        if (threadIdx.x == 0) atomicAdd(&P.counters[4], 1ull);
-        __syncthreads();
-        for (uint32_t i = threadIdx.x; i < kTileDocs; i += kThreads) s_acc[i] = neg_zero;
-        if (threadIdx.x == 0) { sh.touched_n = 0; sh.overflow = 0; }
-        mode = 1;
-        __syncthreads();
-      } else {
-        // which touched docs could still reach the threshold once the non-essential clauses are added
-        const uint32_t n_touched = sh.touched_n;
-        const float ne_bound = sh.ne_bound;
-        for (uint32_t i = threadIdx.x; i < n_touched; i += kThreads) {
-          const uint32_t slot = sh.touched[i];
-          const float est = s_acc[slot];
-          s_acc[slot] = neg_zero;
-          if (est + fabsf(est) * 1e-5f + ne_bound >= theta_f) {
-            const uint32_t j = atomicAdd(&sh.p_n, 1u);
-            if (j < kPromisingCap) { sh.plist[j] = (uint16_t)slot; atomicOr(&sh.pbits[slot >> 5], 1u << (slot & 31u)); }
-            else sh.overflow = 1;
-          }
-        }
-        __syncthreads();
-        const uint32_t p_n = sh.p_n;
-        const bool too_many = sh.overflow != 0;
-        __syncthreads();
-        if (threadIdx.x == 0) {
-          atomicAdd(&P.counters[7], (unsigned long long)sh.touched_n);
-          atomicAdd(&P.counters[too_many ? 5 : (p_n == 0 ? 3 : 6)], too_many ? 1ull : (p_n == 0 ? 1ull : (unsigned long long)p_n));
-          sh.touched_n = 0; sh.overflow = 0;
-        }
-        if (too_many) {
-          for (uint32_t i = threadIdx.x; i < kTileDocs / 32; i += kThreads) sh.pbits[i] = 0;
-          if (threadIdx.x == 0) sh.p_n = 0;
-          mode = 1;
-          __syncthreads();
-        } else if (p_n == 0) {
-          mode = 0;
-        } else {
-          // ---- pruned, stage 2: exact clause-ordered score of the promising docs only -------------------
-          for (uint32_t tt = 0; tt < S.n_lists; ++tt) {
-            const uint32_t blo = sh.blo[buf][tt], bhi = sh.bhi[buf][tt];
-            if (blo <= bhi) {
-              const QList ql = P.qlists[S.lists_base + tt];
-              const ListDesc L = P.lists[ql.list_id];
-              const Scorer scr = make_scorer(P, ql);
-              for (uint32_t b = blo + warp; b <= bhi; b += kWarps) {
-                // does this block's doc range hold a promising doc?
-                const uint32_t last = __ldg(L.last_doc + b);
-                const uint32_t prev = b ? __ldg(L.last_doc + b - 1) : 0u;
-                bool mine = false;
-                for (uint32_t i = lane; i < p_n; i += 32) {
-                  const uint32_t d = lo + sh.plist[i];
-                  mine |= (d <= last) && (b == 0 || d > prev);
-                }
-                if (__ballot_sync(kFull, mine) == 0) continue;
-                uint32_t doc[4], tf[4];
-                decode_block(L, b, lane, doc, tf);
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                  if (doc[i] >= lo && doc[i] < hi) {
-                    const uint32_t slot = doc[i] - lo;
-                    if ((sh.pbits[slot >> 5] >> (slot & 31u)) & 1u) {
-                      const float sc = bm25_score(scr, L.fieldnorm, doc[i], tf[i]);
-                      s_acc[slot] = __fadd_rn(s_acc[slot], sc);
-                    }
-                  }
-                }
-              }
-            }
-            __syncthreads();  // clause order is the f32 summation order
-          }
-          for (uint32_t base = 0; base < p_n; base += kThreads) {
-            const uint32_t i = base + threadIdx.x;
-            bool pass = false;
-            unsigned long long key = 0;
-            if (i < p_n) {
-              const uint32_t slot = sh.plist[i];
-              const float v = s_acc[slot];
-              s_acc[slot] = neg_zero;
-              sh.pbits[slot >> 5] = 0;  // every bit of that word belongs to a promising slot being reset
-              const uint32_t d = lo + slot;
-              key = make_key(v, d);
-              pass = __float_as_uint(v) != 0x80000000u && key >= theta;
-              if (pass && S.alive) pass = is_alive(S.alive, d);
-            }
-            topk_push(T, pass, key, lane);
-          }
-          if (threadIdx.x == 0) sh.p_n = 0;
-          topk_round_end(T, Q.k, &qs->theta);
-          mode = 3;  // done
-        }
-      }
-    }
-
-    if (mode == 1) {
-      // ---- exhaustive accumulate -----------------------------------------------------------------------
+    if (!skip) {
+      // ---- accumulate ----------------------------------------------------------------------------------
       // fieldnorm bytes of the window: one coalesced 16-byte row per thread pair instead of a byte gather per posting
       if (staged_fn) {
         const uint4* src = reinterpret_cast<const uint4*>(S.fieldnorm + lo);
@@ -666,7 +518,7 @@ __global__ void __launch_bounds__(kThreads, 3) k_or(const BatchParams P, uint32_
       or_tile_ranges(P, S, sh, buf ^ 1, tile + 1, warp, lane);
     }
 
-    if (mode == 1) {
+    if (!skip) {
       // harvest: count what passes, then push in one go when it fits.
       // A float compare against the threshold score rejects nearly every slot (untouched slots hold
       // -0.0, which is below any positive threshold); the exact key test runs only on the survivors.
@@ -751,6 +603,8 @@ constexpr uint32_t kMaxCached = 6;
 constexpr uint32_t kStripWarps = 4;
 constexpr uint32_t kStripThreads = kStripWarps * 32;
 constexpr uint32_t kStripMaxLists = 8;
+constexpr uint32_t kStripNeDiv = 8;    // clauses with >= 1 posting per this many docs may turn non-essential
+constexpr uint32_t kStripNeDiv2 = 64;  // ...and the densest clause of a union without such a clause, under this looser bound
 constexpr uint32_t kStripMaxK = 128;
 constexpr uint32_t kNoDoc = 0xFFFFFFFFu;
 
@@ -883,7 +737,7 @@ __global__ void __launch_bounds__(kStripThreads) k_or_strip(const BatchParams P,
   const uint32_t w_end = U.begin + (uint32_t)(((unsigned long long)n_win * (warp + 1)) / kStripWarps);
   for (uint32_t i = lane; i < kWin; i += 32) W.acc[i] = neg_zero;
   const bool staged_fn = (S.flags & 1u) && S.fieldnorm != nullptr;
-  const bool prunable = (S.flags & 2u) != 0 && P.strip_prune != 0;  // every weight finite and >= 0
+  const bool prunable = (S.flags & 2u) != 0;  // every weight finite and >= 0
   uint32_t thick_mask = 0;
   uint32_t n_e_min = 0;  // only the thick clauses at the end of the list may turn non-essential: thin ones are cheap to
                          // apply and every clause kept essential tightens the cold-window test
@@ -908,11 +762,11 @@ __global__ void __launch_bounds__(kStripThreads) k_or_strip(const BatchParams P,
       }
     }
     __syncwarp();
-    {  // a clause may turn non-essential when it has at least one posting per ne_div docs (thick clauses: 1 per 8)
+    {  // a clause may turn non-essential when it has at least one posting per kStripNeDiv docs
       n_e_min = S.n_lists;
-      while (n_e_min > 0 && (unsigned long long)s_list[n_e_min - 1u].doc_freq * P.strip_ne_div >= S.max_doc) --n_e_min;
-      // no such clause: the single densest one may still go if it is dense enough to matter (strip_ne_div2)
-      if (n_e_min == S.n_lists && n_e_min > 1 && (unsigned long long)s_list[n_e_min - 1u].doc_freq * P.strip_ne_div2 >= S.max_doc) --n_e_min;
+      while (n_e_min > 0 && (unsigned long long)s_list[n_e_min - 1u].doc_freq * kStripNeDiv >= S.max_doc) --n_e_min;
+      // no such clause: the single densest one may still go if it is dense enough to matter (kStripNeDiv2)
+      if (n_e_min == S.n_lists && n_e_min > 1 && (unsigned long long)s_list[n_e_min - 1u].doc_freq * kStripNeDiv2 >= S.max_doc) --n_e_min;
     }
     // ---- the windows ---------------------------------------------------------------------------------------
     uint32_t since_refresh = 0;
@@ -1161,329 +1015,6 @@ __global__ void __launch_bounds__(kStripThreads) k_or_strip(const BatchParams P,
       c.pad = 0;
       P.cands[Q.cand_base + base + i] = c;
     }
-  }
-}
-
-// ---- union, pipelined form: TMA bulk copies + mbarrier ring ------------------------------------------------------
-// ncu showed k_or latency bound (about one block per warp in flight, IPC ~1 per SM).  Here a PRODUCER warp walks the
-// block tables of all clauses, one doc-id window after the other, and streams every packed block the window needs
-// into a shared-memory ring with cp.async.bulk (TMA), many blocks and several windows ahead of the 8 CONSUMER warps,
-// which only ever touch shared memory: wait on the slot's mbarrier, pull their vectors, decode, score, add in clause
-// order (named barrier among the consumers between clauses), harvest.  Bytes in flight per SM go from a few hundred
-// to tens of KB.  The window's fieldnorm bytes arrive the same way.
-constexpr uint32_t kPipeSlots = 24;         // ring slots of 1 KB (a block is at most 63 vectors = 1008 B)
-constexpr uint32_t kPipeSlotBytes = 1024 + 16;
-constexpr uint32_t kPipeThreads = kThreads + 32;  // 8 consumer warps + 1 producer warp
-constexpr uint32_t kPipeMaxLists = 8;
-constexpr uint32_t kPipeBatch = 16;          // blocks decoded in parallel before the ordered add (<= kPipeSlots - 8)
-
-struct PipeWindow {  // written by the producer, read by the consumers
-  uint32_t lo, hi, any, pad;
-  uint32_t first[kPipeMaxLists];  // ring item number of the clause's first block in this window
-  uint32_t cnt[kPipeMaxLists];    // how many blocks of the clause overlap the window
-};
-struct PipeShared {
-  unsigned long long full[kPipeSlots], empty[kPipeSlots];
-  unsigned long long win_full[2], win_empty[2];
-  uint2 desc[kPipeSlots];  // .x meta (0xFFFFFFFF: VInt tail, no bytes), .y last doc of the previous block, low bit of block index in... see below
-  uint32_t blk[kPipeSlots]; // block ordinal (needed for the tail pseudo block)
-  PipeWindow win[2];
-};
-__host__ __device__ constexpr size_t pipe_smem_bytes() {
-  return kTileDocs * sizeof(float) + 2 * kTileDocs + kPipeSlots * kPipeSlotBytes;
-}
-
-__device__ __forceinline__ uint32_t smem_u32(const void* p) { return (uint32_t)__cvta_generic_to_shared(p); }
-__device__ __forceinline__ void mbar_init(unsigned long long* bar, uint32_t count) {
-  asm volatile("mbarrier.init.shared::cta.b64 [%0], %1;" ::"r"(smem_u32(bar)), "r"(count) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive(unsigned long long* bar) {
-  asm volatile("mbarrier.arrive.shared::cta.b64 _, [%0];" ::"r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void mbar_arrive_expect_tx(unsigned long long* bar, uint32_t bytes) {
-  asm volatile("mbarrier.arrive.expect_tx.shared::cta.b64 _, [%0], %1;" ::"r"(smem_u32(bar)), "r"(bytes) : "memory");
-}
-__device__ __forceinline__ bool mbar_try_wait(unsigned long long* bar, uint32_t parity) {
-  uint32_t ok;
-  asm volatile("{\n\t.reg .pred p;\n\tmbarrier.try_wait.parity.shared::cta.b64 p, [%1], %2;\n\tselp.b32 %0, 1, 0, p;\n\t}"
-               : "=r"(ok) : "r"(smem_u32(bar)), "r"(parity) : "memory");
-  return ok != 0;
-}
-// A wait that can never hang the device: a protocol error traps after ~2^26 polls instead of spinning for ever.
-__device__ __forceinline__ void mbar_wait(unsigned long long* bar, uint32_t parity) {
-  uint32_t spins = 0;
-  while (!mbar_try_wait(bar, parity)) {
-    if (++spins > (1u << 22)) __trap();
-  }
-}
-__device__ __forceinline__ void bulk_g2s(void* dst, const void* src, uint32_t bytes, unsigned long long* bar) {
-  asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];"
-               ::"r"(smem_u32(dst)), "l"(src), "r"(bytes), "r"(smem_u32(bar)) : "memory");
-}
-__device__ __forceinline__ void pipe_consumer_sync() { asm volatile("bar.sync 1, 256;" ::: "memory"); }
-
-__global__ void __launch_bounds__(kPipeThreads, 2) k_or_pipe(const BatchParams P, uint32_t unit_base) {
-  extern __shared__ __align__(16) unsigned char s_raw[];
-  float* s_acc = reinterpret_cast<float*>(s_raw);                                  // [kTileDocs]
-  uint8_t* s_fn = s_raw + kTileDocs * sizeof(float);                               // [2][kTileDocs]
-  unsigned char* s_ring = s_fn + 2 * kTileDocs;                                    // [kPipeSlots][kPipeSlotBytes]
-  __shared__ CtaTopK s_top;
-  __shared__ PipeShared ps;
-  __shared__ ListDesc s_list[kPipeMaxLists];
-  __shared__ QList s_ql[kPipeMaxLists];
-  const Unit U = P.units[unit_base + blockIdx.x];
-  const QSeg S = P.qsegs[U.qseg];
-  const DQuery Q = P.queries[S.query];
-  QState* qs = P.qstate + S.query;
-  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
-  const bool staged_fn = (S.flags & 1u) && S.fieldnorm != nullptr;
-  const float neg_zero = __uint_as_float(0x80000000u);
-  if (threadIdx.x < S.n_lists) {
-    s_ql[threadIdx.x] = P.qlists[S.lists_base + threadIdx.x];
-    s_list[threadIdx.x] = P.lists[s_ql[threadIdx.x].list_id];
-  }
-  if (threadIdx.x == 0) {
-    for (uint32_t i = 0; i < kPipeSlots; ++i) { mbar_init(&ps.full[i], 1); mbar_init(&ps.empty[i], 1); }
-    for (uint32_t i = 0; i < 2; ++i) { mbar_init(&ps.win_full[i], 1); mbar_init(&ps.win_empty[i], kWarps); }
-    asm volatile("fence.mbarrier_init.release.cluster;" ::: "memory");
-    s_top.count = 0; s_top.theta = (unsigned long long)qs->theta << 32;
-  }
-  for (uint32_t i = threadIdx.x; i < kTileDocs; i += kPipeThreads) s_acc[i] = neg_zero;
-  __syncthreads();
-  const uint32_t n_windows = U.end - U.begin;
-
-  if (warp == kWarps) {
-    // =========================== producer ======================================================================
-    __shared__ uint32_t p_cur[kPipeMaxLists], p_blo[kPipeMaxLists], p_cnt[kPipeMaxLists];
-    if (lane < kPipeMaxLists) p_cur[lane] = 0;
-    __syncwarp();
-    uint32_t n_item = 0;  // ring item counter
-    for (uint32_t wi = 0; wi < n_windows; ++wi) {
-      const uint32_t tile = U.begin + wi;
-      const uint32_t lo = tile * kTileDocs, hi = min(lo + kTileDocs, S.max_doc);
-      const uint32_t buf = wi & 1u;
-      if (wi >= 2) mbar_wait(&ps.win_empty[buf], ((wi >> 1) - 1u) & 1u);  // the consumers are done with this buffer's previous window
-      // where every clause stands in this window
-      uint32_t total = 0;
-      for (uint32_t t = 0; t < S.n_lists; ++t) {
-        const ListDesc& L = s_list[t];
-        uint32_t blo = 0, cnt = 0;
-        const uint32_t j_lo = first_block_ge(L.last_doc, p_cur[t], L.n_total, lo, lane);
-        if (j_lo < L.n_total) {
-          uint32_t j_hi = first_block_ge(L.last_doc, j_lo, L.n_total, hi - 1u, lane);
-          if (j_hi >= L.n_total) j_hi = L.n_total - 1u;
-          blo = j_lo; cnt = j_hi - j_lo + 1u;
-        }
-        __syncwarp();
-        if (lane == 0) { p_cur[t] = j_lo; p_blo[t] = blo; p_cnt[t] = cnt; }
-        total += cnt;
-      }
-      __syncwarp();
-      if (lane == 0) {
-        PipeWindow& w = ps.win[buf];
-        w.lo = lo; w.hi = hi; w.any = total;
-        uint32_t n = n_item;
-        for (uint32_t t = 0; t < kPipeMaxLists; ++t) {
-          const uint32_t c = t < S.n_lists ? p_cnt[t] : 0u;
-          w.first[t] = n; w.cnt[t] = c; n += c;
-        }
-        if (staged_fn && total) {
-          mbar_arrive_expect_tx(&ps.win_full[buf], kTileDocs);
-          bulk_g2s(s_fn + buf * kTileDocs, S.fieldnorm + lo, kTileDocs, &ps.win_full[buf]);
-        } else {
-          mbar_arrive(&ps.win_full[buf]);
-        }
-      }
-      __syncwarp();
-      for (uint32_t t = 0; t < S.n_lists; ++t) {
-        const ListDesc& L = s_list[t];
-        const uint32_t cnt = p_cnt[t], blo = p_blo[t];
-        // 16 blocks per step, one lane per block.  A slot frees up only when the consumers have added a whole BATCH,
-        // and that batch may contain blocks of this very step, so a lane must never make another lane wait: every
-        // lane polls its slot once per turn and issues the moment it is free.
-        for (uint32_t base = 0; base < cnt; base += 16) {
-          const uint32_t i = base + lane;
-          bool pending = lane < 16 && i < cnt;
-          const uint32_t b = blo + i;
-          const uint32_t n = n_item + i;
-          const uint32_t slot = n % kPipeSlots, round = n / kPipeSlots;
-          uint32_t turns = 0;
-          while (__ballot_sync(kFull, pending)) {
-            if (pending && mbar_try_wait(&ps.empty[slot], (round & 1u) ^ 1u)) {  // free (true at once in the first round)
-              pending = false;
-              ps.blk[slot] = b;
-              if (b >= L.n_blocks) {  // VInt tail: already decoded in global memory, nothing to copy
-                ps.desc[slot] = make_uint2(0xFFFFFFFFu, 0u);
-                mbar_arrive(&ps.full[slot]);
-              } else {
-                const uint4 rec = __ldg(L.tab4 + b);
-                ps.desc[slot] = make_uint2(rec.z, rec.w == 0xFFFFFFFFu ? 0u : rec.w);
-                const uint32_t bytes = 16u * ((rec.z & 31u) + (L.has_freq ? ((rec.z >> 8) & 63u) : 0u));
-                if (bytes) {
-                  mbar_arrive_expect_tx(&ps.full[slot], bytes);
-                  bulk_g2s(s_ring + slot * kPipeSlotBytes, L.blocks + rec.y, bytes, &ps.full[slot]);
-                } else {
-                  mbar_arrive(&ps.full[slot]);
-                }
-              }
-            }
-            if (++turns > (1u << 24)) __trap();  // protocol error: fail loudly instead of hanging the device
-          }
-        }
-        n_item += cnt;
-      }
-    }
-  } else {
-    // =========================== consumers =====================================================================
-    const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, P.counters, 1u, (unsigned)kThreads};
-    unsigned int theta_g_seen = 0;
-    for (uint32_t wi = 0; wi < n_windows; ++wi) {
-      const uint32_t buf = wi & 1u;
-      mbar_wait(&ps.win_full[buf], (wi >> 1) & 1u);
-      const PipeWindow& w = ps.win[buf];
-      const uint32_t lo = w.lo, hi = w.hi;
-      const bool any = w.any != 0;
-      if (threadIdx.x == 0) {
-        const unsigned long long g = (unsigned long long)theta_g_seen << 32;
-        if (g > s_top.theta) s_top.theta = g;
-        theta_g_seen = *(volatile unsigned int*)&qs->theta;
-      }
-      if (any) {
-        const uint8_t* fn_tile = s_fn + buf * kTileDocs;
-        // The window's blocks are taken in batches of kPipeBatch (clause order).  Phase 1, no ordering needed: the
-        // warps decode and SCORE the batch's blocks in parallel and park (slot, score) pairs in the block's own ring
-        // slot.  Phase 2, ordered: clause by clause the pairs are added to the score slots (a few instructions per
-        // posting), with a consumer barrier between clauses.  Only the cheap phase is serialised by the clause order.
-        const uint32_t n0 = w.first[0];
-        const uint32_t total = w.any;
-        for (uint32_t done = 0; done < total; done += kPipeBatch) {
-          const uint32_t nb = min(total - done, kPipeBatch);
-          for (uint32_t j = done + warp; j < done + nb; j += kWarps) {
-            uint32_t t = 0;
-            while (t + 1 < S.n_lists && j >= w.first[t + 1] - n0) ++t;  // clause of item j (first[] is non-decreasing)
-            const ListDesc& L = s_list[t];
-            const Scorer scr = make_scorer(P, s_ql[t]);
-            const uint32_t n = n0 + j;
-            const uint32_t slot = n % kPipeSlots, round = n / kPipeSlots;
-            mbar_wait(&ps.full[slot], round & 1u);
-            const uint2 d = ps.desc[slot];
-            const uint32_t b = ps.blk[slot];
-            unsigned char* sbase = s_ring + slot * kPipeSlotBytes;
-            BlockFetch f;
-            f.meta = d.x; f.prev = d.y;
-            if (d.x != 0xFFFFFFFFu) {
-              const uint32_t db = d.x & 31u, tb = (d.x >> 8) & 63u;
-              const uint4* v = reinterpret_cast<const uint4*>(sbase);
-              const uint32_t wd = (lane * db) >> 5;
-              f.dlo = v[wd]; f.dhi = v[wd + 1];
-              if (L.has_freq) { const uint32_t wt = db + ((lane * tb) >> 5); f.tlo = v[wt]; f.thi = v[wt + 1]; }
-            }
-            uint32_t doc[4], tf[4];
-            fetch_decode(L, b, f, lane, doc, tf);
-            __syncwarp();  // every lane has its vectors: the slot's bytes can be overwritten by the pairs
-            uint16_t* pslot = reinterpret_cast<uint16_t*>(sbase);
-            float* pscore = reinterpret_cast<float*>(sbase + 256);
-#pragma unroll
-            for (int k4 = 0; k4 < 4; ++k4) {
-              uint16_t s16 = 0xFFFFu;
-              float sc = 0.0f;
-              if (doc[k4] >= lo && doc[k4] < hi) {
-                const uint32_t slot_d = doc[k4] - lo;
-                const uint32_t id = staged_fn ? (uint32_t)fn_tile[slot_d] : (L.fieldnorm ? (uint32_t)__ldg(L.fieldnorm + doc[k4]) : 1u);
-                sc = bm25_score_id(scr, id, tf[k4]);
-                s16 = (uint16_t)slot_d;
-              }
-              pslot[lane * 4 + k4] = s16;
-              pscore[lane * 4 + k4] = sc;
-            }
-          }
-          pipe_consumer_sync();  // all pairs of the batch are parked
-          for (uint32_t t = 0; t < S.n_lists; ++t) {
-            if (w.cnt[t] == 0) continue;
-            const uint32_t c_lo = w.first[t] - n0, c_hi = c_lo + w.cnt[t];
-            const uint32_t j_lo = max(c_lo, done), j_hi = min(c_hi, done + nb);
-            if (j_lo >= j_hi) continue;  // clause not in this batch (uniform across the consumers)
-            for (uint32_t j = j_lo + ((warp + kWarps - (j_lo & (kWarps - 1))) & (kWarps - 1)); j < j_hi; j += kWarps) {
-              // j % kWarps == warp: the warp that parked the pairs also adds them and then frees the slot
-              const uint32_t n = n0 + j;
-              const uint32_t slot = n % kPipeSlots;
-              const unsigned char* sbase = s_ring + slot * kPipeSlotBytes;
-              const ushort4 s4 = reinterpret_cast<const ushort4*>(sbase)[lane];
-              const float4 v4 = reinterpret_cast<const float4*>(sbase + 256)[lane];
-              if (s4.x != 0xFFFFu) s_acc[s4.x] = __fadd_rn(s_acc[s4.x], v4.x);
-              if (s4.y != 0xFFFFu) s_acc[s4.y] = __fadd_rn(s_acc[s4.y], v4.y);
-              if (s4.z != 0xFFFFu) s_acc[s4.z] = __fadd_rn(s_acc[s4.z], v4.z);
-              if (s4.w != 0xFFFFu) s_acc[s4.w] = __fadd_rn(s_acc[s4.w], v4.w);
-              __syncwarp();
-              if (lane == 0) mbar_arrive(&ps.empty[slot]);
-            }
-            pipe_consumer_sync();  // clause order is the f32 summation order
-          }
-        }
-        // ---- harvest (same as k_or, consumers only) -----------------------------------------------------------
-        const unsigned long long theta = *T.theta;
-        const float theta_f = threshold_score((uint32_t)(theta >> 32));
-        uint32_t passmask = 0;
-#pragma unroll 1
-        for (int j = 0; j < (int)(kTileDocs / (kThreads * 4)); ++j) {
-          const uint32_t idx = (j * kThreads + threadIdx.x) * 4;
-          const float4 v = *reinterpret_cast<const float4*>(s_acc + idx);
-          if (v.x >= theta_f || v.y >= theta_f || v.z >= theta_f || v.w >= theta_f) {
-            const float vv[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-              const uint32_t dd = lo + idx + c;
-              bool pass = vv[c] >= theta_f && __float_as_uint(vv[c]) != 0x80000000u && make_key(vv[c], dd) >= theta;
-              if (pass && S.alive) pass = is_alive(S.alive, dd);
-              passmask |= pass ? (1u << (j * 4 + c)) : 0u;
-            }
-          }
-        }
-        // room check: the buffer keeps at most kCap - kRoundMargin keys between windows, a window adds at most... see below
-        const uint32_t wsum = __reduce_add_sync(kFull, (uint32_t)__popc(passmask));
-        __shared__ uint32_t s_npass;
-        if (threadIdx.x == 0) s_npass = 0;
-        pipe_consumer_sync();
-        if (lane == 0 && wsum) atomicAdd(&s_npass, wsum);
-        pipe_consumer_sync();
-        const bool fits = *T.count + s_npass <= kCap;
-        pipe_consumer_sync();  // every consumer has read the count before anyone starts pushing (the branch must be uniform)
-        if (fits) {
-#pragma unroll 1
-          for (int j = 0; j < (int)(kTileDocs / (kThreads * 4)); ++j) {
-            const uint32_t idx = (j * kThreads + threadIdx.x) * 4;
-            const uint32_t sub = (passmask >> (j * 4)) & 15u;
-            if (__ballot_sync(kFull, sub != 0)) {
-              const float4 v = *reinterpret_cast<const float4*>(s_acc + idx);
-              const float vv[4] = {v.x, v.y, v.z, v.w};
-#pragma unroll
-              for (int c = 0; c < 4; ++c) topk_push(T, (sub >> c) & 1u, make_key(vv[c], lo + idx + c), lane);
-            }
-            *reinterpret_cast<float4*>(s_acc + idx) = make_float4(neg_zero, neg_zero, neg_zero, neg_zero);
-          }
-          topk_round_end(T, Q.k, &qs->theta);
-        } else {  // cold start: go in rounds with compaction between
-          topk_round_end(T, Q.k, &qs->theta);
-#pragma unroll 1
-          for (int j = 0; j < (int)(kTileDocs / (kThreads * 4)); ++j) {
-            const uint32_t idx = (j * kThreads + threadIdx.x) * 4;
-            const float4 v = *reinterpret_cast<const float4*>(s_acc + idx);
-            const float vv[4] = {v.x, v.y, v.z, v.w};
-            const unsigned long long th = *T.theta;
-#pragma unroll
-            for (int c = 0; c < 4; ++c) {
-              const unsigned long long key = make_key(vv[c], lo + idx + c);
-              topk_push(T, ((passmask >> (j * 4 + c)) & 1u) && key >= th, key, lane);
-            }
-            *reinterpret_cast<float4*>(s_acc + idx) = make_float4(neg_zero, neg_zero, neg_zero, neg_zero);
-            topk_round_end(T, Q.k, &qs->theta);
-          }
-        }
-      }
-      __syncwarp();
-      if (lane == 0) mbar_arrive(&ps.win_empty[buf]);  // this warp no longer reads the window's table or fieldnorms
-    }
-    topk_flush(T, Q, qs, P.cands, S.segment_ord);
   }
 }
 

@@ -286,7 +286,7 @@ __global__ void __launch_bounds__(kPhraseThreads, 5) k_phrase(const BatchParams 
   const Scorer sc = make_scorer(P, ql0);  // the phrase's single Bm25Weight
   if (threadIdx.x == 0) { s_top.count = 0; s_top.theta = (unsigned long long)qs->theta << 32; }
   __syncthreads();
-  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, P.counters, 0u, (unsigned)kPhraseThreads};
+  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, (unsigned)kPhraseThreads};
   for (uint32_t r = U.begin; r < U.end; r += kPhraseWarps) {
     const uint32_t b = r + warp;
     if (b < U.end) {

@@ -33,7 +33,7 @@ def _ctx_with_env(**env):
 
 
 # every test runs on both union engines: "tile" = the shared-decode tile engine (k_score_lists + k_tile, the default),
-# "legacy" = the per-query kernels (k_or_strip / k_or_pipe / k_or) that the tile engine falls back to
+# "legacy" = the per-query kernels (k_or_strip, and k_or for > 8 clauses or k > 128) that the tile engine falls back to
 @pytest.fixture(scope="module", params=["tile", "legacy"])
 def ctx(request):
     # (TQ_TILE_TERMS=1: single-term batches stay on the tile engine here; the default rule has a test of its own)
@@ -374,8 +374,9 @@ def test_synth_mixed_batch(ctx, synth):
 
 
 def test_synth_union_pruning_is_exact(ctx, synth):
-    """Unions of dense and rare terms with small k make k_or switch to its MaxScore-pruned route after
-    the first windows; the result must stay identical to the exhaustive oracle, hit for hit."""
+    """Unions of dense and rare terms with small k: the tile engine prunes on its per-tile maxima, and on the legacy
+    engine k_or_strip splits off the non-essential clauses (MaxScore) and runs its threshold rounds; the result must
+    stay identical to the exhaustive oracle, hit for hit."""
     ix, oi, base = synth
     queries = []
     for k in (1, 3, 10, 50):
@@ -522,6 +523,8 @@ def test_tile_engine_is_what_runs(ctx, synth):
         assert st["units_or"] == 0  # no per-query union kernel ran
     else:
         assert st["tile_groups"] == 0 and st["units_or"] > 0
+        # k <= 128: k_or_strip; the k = 1000 queries take k_or
+        assert st["units_or"] > st["units_or_strip"] > 0
 
 
 @pytest.mark.parametrize("hook", [dict(TQ_TILE_PCAP=64), dict(TQ_TILE_CAND_FLOOR=4), dict(TQ_TILE_SAMPLE_DIV=0, TQ_TILE_CAND_FLOOR=64)])
