@@ -57,7 +57,9 @@ extern "C" {
  * one).  A doc matches when every MUST group has a clause that lists it, at least `min_should_match` SHOULD clauses list
  * it (at least one when there is no MUST group: boolean_weight.rs:354-366), and no MUST_NOT clause lists it (Exclude).
  * Score = (sum over the MUST groups, ascending cost, of the sum of their matching clauses) + (sum of the matching SHOULD
- * clauses) -- Intersection::score / RequiredOptionalScorer::score (intersection.rs:325-329, reqopt_scorer.rs:78-94). */
+ * clauses) -- Intersection::score / RequiredOptionalScorer::score (intersection.rs:325-329, reqopt_scorer.rs:78-94).
+ * Runs on both engines with the same rows: the tile engine when the query fits a tile group, else (and with TQ_TILE=0, and
+ * when an overflowing tile-engine run is repeated) the per-query kernel k_bool. */
 #define TQ_OP_BOOL 4
 #define TQ_OCCUR_SHOULD 0
 #define TQ_OCCUR_MUST 1
@@ -171,6 +173,8 @@ typedef struct {
   uint64_t tile_counters[8];    /* cumulative, with TQ_TILE_COUNTERS=1: (query, tile) pairs seen / skipped / light / heavy,
                                    essential postings applied, docs completed, docs at or above the threshold;
                                    [7] (always): dynamic shared memory bytes of a k_tile CTA of the last prepared group */
+  uint64_t units_bool;          /* CTAs of k_bool (TQ_OP_BOOL queries on the per-query kernels) */
+  float bool_ms;                /* device time of k_bool */
 } tq_stats;
 
 /* ---- context ------------------------------------------------------------------------- */

@@ -119,6 +119,8 @@ class Stats(C.Structure):
         ("tile_scratch_bytes", C.c_uint64),
         ("tile_fallbacks", C.c_uint64),
         ("tile_counters", C.c_uint64 * 8),
+        ("units_bool", C.c_uint64),
+        ("bool_ms", C.c_float),
     ]
 
 

@@ -56,7 +56,7 @@ struct QList {  // one clause of one query in one segment
   uint32_t list_id;
   float weight;        // Bm25Weight.weight
   uint32_t cache_idx;  // which 256-entry tf-norm table
-  uint32_t pad;
+  uint32_t pad;        // k_or_strip: thin-clause cache slot; k_bool: role | group << 2
 };
 struct QSeg {  // one (query, segment): what Collector::collect_segment sees
   uint32_t query;
@@ -64,7 +64,8 @@ struct QSeg {  // one (query, segment): what Collector::collect_segment sees
   uint32_t n_lists;
   uint32_t max_doc;
   uint32_t segment_ord;
-  uint32_t flags;        // bit 0: every clause reads the same fieldnorm array (`fieldnorm` below)
+  uint32_t flags;        // bit 0: every clause reads the same fieldnorm array (`fieldnorm` below), bit 1: every weight finite and >= 0;
+                         // k_bool: [8:16) MUST groups, [16:24) SHOULD clauses needed
   const uint8_t* alive;  // alive bitset bytes or null
   const uint8_t* fieldnorm;  // shared fieldnorm ids (padded to a multiple of kTileDocs) when flags&1
 };

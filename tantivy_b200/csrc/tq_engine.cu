@@ -194,8 +194,8 @@ struct tq_batch {
   BatchParams params{};
   size_t desc_bytes = 0;
   uint32_t nq = 0, kmax = 0;
-  uint32_t n_units[8] = {0, 0, 0, 0, 0, 0, 0, 0};  // term, and, or (window kernel), or (strip kernel), strip threshold rounds 1..3, phrase
-  uint32_t unit_base[8] = {0, 0, 0, 0, 0, 0, 0, 0};
+  uint32_t n_units[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};  // term, and, or (window kernel), or (strip kernel), strip threshold rounds 1..3, phrase, mixed boolean
+  uint32_t unit_base[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};
   uint32_t phrase_ct = 2;                 // most terms of a phrase in the batch (k_phrase's candidate stride)
   const PhraseAux* phrase_aux = nullptr;  // device: per clause of the batch's phrase queries (parallel to qlists)
   uint32_t strip_cached_max = 0;
@@ -271,6 +271,7 @@ int tq_ctx_create(int device, tq_ctx** out) {
   if (err == cudaSuccess) err = cudaMemset(c->d_counters, 0, 16 * sizeof(unsigned long long));
   if (err == cudaSuccess) err = cudaStreamCreateWithFlags(&c->build_stream, cudaStreamNonBlocking);
   if (err == cudaSuccess) err = cudaFuncSetAttribute(k_or, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kOrDynSmem);
+  if (err == cudaSuccess) err = cudaFuncSetAttribute(k_bool, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)kBoolDynSmem);  // (+ its static smem: > 48 KB)
   if (err == cudaSuccess) err = cudaFuncSetAttribute(k_or_strip, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)strip_smem_bytes(kMaxCached));
   if (err == cudaSuccess) err = cudaFuncSetAttribute(k_tile, cudaFuncAttributeMaxDynamicSharedMemorySize, 200 * 1024);
   if (err != cudaSuccess) { delete c; return fail(TQ_ERR_CUDA, cudaGetErrorString(err)); }
@@ -635,7 +636,7 @@ struct CacheKey {
 
 // ---- batches ---------------------------------------------------------------------------------------
 // Kernel time by kind: CUDA events recorded on the batch's stream around every launch (group of launches) of that kind.
-enum SpanKind { SPAN_TERM = 0, SPAN_AND, SPAN_OR, SPAN_FINAL, SPAN_SCORE, SPAN_TILE, SPAN_THETA, SPAN_PHRASE, SPAN_KINDS };
+enum SpanKind { SPAN_TERM = 0, SPAN_AND, SPAN_OR, SPAN_FINAL, SPAN_SCORE, SPAN_TILE, SPAN_THETA, SPAN_PHRASE, SPAN_BOOL, SPAN_KINDS };
 
 static int span_begin(tq_batch* b, int kind, cudaStream_t on = nullptr) {
   if (b->n_spans == b->spans.size()) {
@@ -667,6 +668,7 @@ static void collect_times(tq_batch* b) {
   b->stats.tile_ms = by_kind[SPAN_TILE];
   b->stats.theta_ms = by_kind[SPAN_THETA];
   b->stats.phrase_ms = by_kind[SPAN_PHRASE];
+  b->stats.bool_ms = by_kind[SPAN_BOOL];
 }
 
 static tq_batch* acquire_batch(tq_ctx* c) {
@@ -918,7 +920,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
 
   std::vector<QList> qlists;
   std::vector<QSeg> qsegs;
-  std::vector<Unit> units[8];
+  std::vector<Unit> units[9];
   std::vector<PhraseAux> qaux;  // parallel to qlists once a phrase query shows up
   std::vector<PendingPos> pending_pos;
   std::vector<DQuery> dq(nq);
@@ -930,7 +932,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   size_t n_cands = 0;
   std::vector<int> qseg_op;
   std::vector<uint32_t> qseg_total;
-  uint32_t n_qsegs_op[4] = {0, 0, 0, 0};
+  uint32_t n_qsegs_op[9] = {0, 0, 0, 0, 0, 0, 0, 0, 0};  // (query, segment) pairs per unit class
   std::vector<char> qseg_sample;  // strip pairs that get a threshold sample pass (MaxScore can then skip their dense clauses)
   uint32_t strip_cached_max = 0, phrase_ct = 2;
   std::vector<TileGroupBuild> tgroups;
@@ -957,7 +959,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
       if (q.k == 0 || q.k > TQ_MAX_K) return fail(TQ_ERR_INVALID_ARGUMENT, "k must be in 1..TQ_MAX_K");
       if (q.n_terms == 0 || q.n_terms > TQ_MAX_TERMS) return fail(TQ_ERR_INVALID_ARGUMENT, "n_terms must be in 1..TQ_MAX_TERMS");
       const bool is_bool = q.op == TQ_OP_BOOL;
-      if (is_bool && (!tile_on || !q.term_occur)) return fail(!q.term_occur ? TQ_ERR_INVALID_ARGUMENT : TQ_ERR_UNSUPPORTED, "TQ_OP_BOOL needs term_occur and the tile engine (TQ_TILE=1)");
+      if (is_bool && !q.term_occur) return fail(TQ_ERR_INVALID_ARGUMENT, "TQ_OP_BOOL needs term_occur");
       if (q.op != TQ_OP_TERM && q.op != TQ_OP_AND && q.op != TQ_OP_OR && q.op != TQ_OP_PHRASE && !is_bool) return fail(TQ_ERR_INVALID_ARGUMENT, "op");
       if (q.op == TQ_OP_TERM && q.n_terms != 1) return fail(TQ_ERR_INVALID_ARGUMENT, "TQ_OP_TERM takes one term");
       if (!q.weight || (!q.avg_fieldnorm && !q.tf_cache) || (!q.term_segs && q.n_term_segs)) return fail(TQ_ERR_INVALID_ARGUMENT, "query arrays");
@@ -1091,7 +1093,6 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
         }
       }
       if (on_tile) continue;
-      if (op == TQ_OP_BOOL && n_plans) return fail(TQ_ERR_UNSUPPORTED, "TQ_OP_BOOL query does not fit the tile engine's buffers (split the batch / raise TQ_TILE_SCRATCH_MB)");
       for (size_t pi = 0; pi < n_plans; ++pi) {
         SegPlan& sp = plans[pi];
         auto& here = sp.here;
@@ -1105,7 +1106,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
         qs.fieldnorm = sp.uniform_fn ? sp.fn0 : nullptr;
         const bool prunable = sp.prunable && op != TQ_OP_TERM;
         qs.flags = (sp.uniform_fn ? 1u : 0u) | (prunable ? 2u : 0u);
-        int unit_class = op == TQ_OP_PHRASE ? 7 : op;
+        int unit_class = op == TQ_OP_PHRASE ? 7 : (op == TQ_OP_BOOL ? 8 : op);
         if (op == TQ_OP_PHRASE) {
           if (qaux.size() < qlists.size()) qaux.resize(qlists.size(), PhraseAux{0, 0, 0});
           for (auto& h : here) { qaux.push_back(PhraseAux{h.second.pad, h.range_len, q.slop}); h.second.pad = 0; }
@@ -1123,7 +1124,22 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
             unit_class = 3;
           }
         }
-        for (auto& h : here) qlists.push_back(h.second);
+        if (op == TQ_OP_BOOL) {
+          // k_bool: the clauses in bool_structure's order (groups, SHOULD, MUST_NOT); QList.pad = role | group << 2,
+          // QSeg.flags [8:16) = number of groups, [16:24) = SHOULD clauses needed
+          const std::vector<uint16_t>& w = sp.bool_words;
+          const uint32_t ng = w[0], ns = w[2], nn = w[3];
+          qs.flags |= (ng << 8) | ((uint32_t)w[1] << 16);
+          size_t x = 4;
+          for (uint32_t g = 0; g < ng; ++g) {
+            const uint16_t len = w[x++];
+            for (uint16_t e = 0; e < len; ++e) { QList ql = here[w[x++]].second; ql.pad = kBoolMust | (g << 2); qlists.push_back(ql); }
+          }
+          for (uint32_t e = 0; e < ns; ++e) { QList ql = here[w[x++]].second; ql.pad = kBoolShould; qlists.push_back(ql); }
+          for (uint32_t e = 0; e < nn; ++e) { QList ql = here[w[x++]].second; ql.pad = kBoolNot; qlists.push_back(ql); }
+        } else {
+          for (auto& h : here) qlists.push_back(h.second);
+        }
         qs.n_lists = (uint32_t)here.size();
         const uint32_t lead_total = here[0].first / 128u + ((here[0].first % 128u) ? 1u : 0u);
         qsegs.push_back(qs);
@@ -1133,7 +1149,9 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
           for (auto& h : here) any_thick = any_thick || (uint64_t)h.first * std::max(kStripNeDiv, kStripNeDiv2) >= qs.max_doc;
           qseg_sample.push_back(unit_class == 3 && prunable && any_thick);
         }
-        qseg_total.push_back(unit_class == 3 ? (qs.max_doc + kWin - 1) / kWin : (op == TQ_OP_OR ? (qs.max_doc + kTileDocs - 1) / kTileDocs : lead_total));
+        qseg_total.push_back(unit_class == 3 ? (qs.max_doc + kWin - 1) / kWin
+                                             : (op == TQ_OP_OR ? (qs.max_doc + kTileDocs - 1) / kTileDocs
+                                                               : (op == TQ_OP_BOOL ? (qs.max_doc + kBoolDocs - 1) / kBoolDocs : lead_total)));
         ++n_qsegs_op[unit_class == 7 ? TQ_OP_AND : unit_class];
       }
     }
@@ -1144,7 +1162,9 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
     for (size_t s = 0; s < qsegs.size(); ++s) {
       const int op = qseg_op[s];
       const uint32_t total = qseg_total[s];
-      const uint32_t min_per = op == TQ_OP_TERM ? c->term_blocks_per_unit : ((op == TQ_OP_AND || op == 7) ? c->and_blocks_per_unit : (op == 3 ? kStripWarps * 64u : 16u));
+      // (k_bool: 32 of its 4096-doc windows, the docs of k_or's 16 8192-doc windows)
+      const uint32_t min_per = op == TQ_OP_TERM ? c->term_blocks_per_unit
+                                                : ((op == TQ_OP_AND || op == 7) ? c->and_blocks_per_unit : (op == 3 ? kStripWarps * 64u : (op == 8 ? 32u : 16u)));
       const uint32_t n_same = n_qsegs_op[op == 7 ? TQ_OP_AND : op];
       const uint32_t want_units = std::max<uint32_t>(1u, (target_units + n_same - 1) / n_same);
       const uint32_t per = std::max<uint32_t>(min_per, (total + want_units - 1) / want_units);
@@ -1314,7 +1334,8 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   const size_t o_qlists = off; off = align(off + qlists.size() * sizeof(QList));
   const size_t o_qsegs = off; off = align(off + qsegs.size() * sizeof(QSeg));
   const size_t o_qaux = off; off = align(off + qaux.size() * sizeof(PhraseAux));
-  const size_t n_units_total = units[0].size() + units[1].size() + units[2].size() + units[3].size() + units[4].size() + units[5].size() + units[6].size() + units[7].size();
+  const size_t n_units_total = units[0].size() + units[1].size() + units[2].size() + units[3].size() + units[4].size() + units[5].size() + units[6].size() + units[7].size() +
+                               units[8].size();
   b->strip_cached_max = strip_cached_max;
   b->phrase_ct = std::min<uint32_t>(phrase_ct, kPhraseMaxTerms);
   const size_t o_units = off; off = align(off + n_units_total * sizeof(Unit));
@@ -1366,7 +1387,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   {
     Unit* u = reinterpret_cast<Unit*>(b->pin.p + o_units);
     uint32_t base = 0;
-    for (int op = 0; op < 8; ++op) {
+    for (int op = 0; op < 9; ++op) {
       b->unit_base[op] = base;
       b->n_units[op] = (uint32_t)units[op].size();
       if (!units[op].empty()) memcpy(u + base, units[op].data(), units[op].size() * sizeof(Unit));
@@ -1533,6 +1554,7 @@ static int batch_prepare_impl(tq_ctx* c, const tq_query* queries, size_t nq, boo
   b->stats.bytes_term = op_bytes[0]; b->stats.bytes_and = op_bytes[1]; b->stats.bytes_or = op_bytes[2];
   b->stats.units_tile = tile_units;
   b->stats.units_phrase = units[7].size();
+  b->stats.units_bool = units[8].size();
   b->stats.tile_groups = b->groups.size();
   b->stats.tile_postings = tile_postings;
   for (auto& tg : tgroups) b->stats.tile_list_bytes += tg.list_bytes;
@@ -1606,6 +1628,11 @@ static int run_phase(tq_batch* b, int phase) {
     if (b->n_units[TQ_OP_OR]) {
       const int sp = span_begin(b, SPAN_OR);
       k_or<<<b->n_units[TQ_OP_OR], kThreads, kOrDynSmem, b->stream>>>(P, b->unit_base[TQ_OP_OR]); ++launches;
+      span_end(b, sp);
+    }
+    if (b->n_units[8]) {
+      const int sp = span_begin(b, SPAN_BOOL);
+      k_bool<<<b->n_units[8], kThreads, kBoolDynSmem, b->stream>>>(P, b->unit_base[8]); ++launches;
       span_end(b, sp);
     }
     if (tiles) {  // K1 + K2 once for every distinct list of the batch

@@ -9,6 +9,8 @@
 //                   leader first, then secondaries by ascending doc_freq (:27,146-158)
 //   k_or            BufferedUnionScorer's shape (union/buffered_union.rs:63-151): a doc-id window of
 //                   score slots in shared memory, clauses accumulated in clause order
+//   k_bool          BooleanWeight::complex_scorer's result set for mixed Occurs (boolean_weight.rs:236-431):
+//                   k_or's windows with per-group presence bitmaps, SHOULD counts and a MUST_NOT mask
 //   k_final         TopBySortKeyCollector::merge_fruits / merge_top_k (sort_key_top_collector.rs:54-95)
 #pragma once
 #include "tq_device.cuh"
@@ -1219,6 +1221,247 @@ __global__ void __launch_bounds__(kThreads) k_count_bool(const CountBoolParams P
     for (int w = 0; w < kWarps; ++w) sum += s_part[w];
     if (sum) atomicAdd(&P.counts[S.query], sum);
   }
+}
+
+// ---- mixed boolean shapes (TQ_OP_BOOL), per query ----------------------------------------------------------------------
+// The per-query form of tile_eval_bool (tq_tile.cuh): BooleanWeight::complex_scorer for term leaves (boolean_weight.rs:236-431),
+// evaluated window by window like k_count_bool matches and k_or scores.  The QSeg's clauses are laid out
+//   MUST groups (ascending cost; each group's clauses by descending weight), SHOULD clauses, MUST_NOT clauses
+// with QList.pad = role | group << 2 and QSeg.flags bits [8:16) = number of groups, [16:24) = SHOULD clauses needed.
+// Per window: each group's clauses are added into a per-doc group score (first match assigned, clause order), folded into the
+// running total (group order) and its presence bits and-ed into the match mask; an empty mask ends the window.  Then the SHOULD
+// clauses (a second sum + per-doc counts), the MUST_NOT clauses (cleared from the mask), and the harvest of k_or.
+// score = ng ? (cnt ? total + ss : total) : ss, the f32 operations and order of tile_eval_bool and of the oracle's bool_for_each.
+constexpr uint32_t kBoolDocs = 4096;  // doc ids per window
+constexpr uint32_t kBoolWords = kBoolDocs / 32u;
+constexpr uint32_t kBoolMust = 0, kBoolShould = 1, kBoolNot = 2;  // QList.pad & 3
+constexpr size_t kBoolDynSmem = 2u * kBoolDocs * sizeof(float) + 2u * kBoolDocs + 2u * kBoolWords * 4u;
+
+struct BoolShared {
+  uint32_t blo[32], bhi[32];  // per clause: block range overlapping the window (blo > bhi: none)
+  uint32_t cur[32];           // per clause: search cursor
+  uint32_t npass;
+  float bound;                // no doc of the segment scores above this (prunable shapes)
+  uint32_t skip;
+};
+
+// Every posting of the clause's blocks [blo, bhi] that falls in [lo, hi): f(slot, score) (kScore: false passes 0).  Warps take
+// the blocks round robin; the next block of a warp travels while this one is scored.
+template <bool kScore, class F>
+__device__ __forceinline__ void bool_for_each_posting(const BatchParams& P, const QList& ql, uint32_t blo, uint32_t bhi, uint32_t lo, uint32_t hi,
+                                                      const uint8_t* s_fn, bool staged_fn, uint32_t warp, uint32_t lane, F f) {
+  if (blo > bhi || blo + warp > bhi) return;
+  const ListDesc L = P.lists[ql.list_id];
+  const Scorer scr = make_scorer(P, ql);
+  BlockFetch fch;
+  fetch_issue(L, blo + warp, lane, fch);
+  for (uint32_t b = blo + warp; b <= bhi; b += kWarps) {
+    uint32_t doc[4], tf[4];
+    fetch_decode(L, b, fch, lane, doc, tf);
+    if (b + kWarps <= bhi) fetch_issue(L, b + kWarps, lane, fch);
+    float sc[4] = {0.f, 0.f, 0.f, 0.f};
+    if (kScore) {
+#pragma unroll
+      for (int i = 0; i < 4; ++i) {
+        if (doc[i] >= lo && doc[i] < hi) {
+          const uint32_t id = staged_fn ? (uint32_t)s_fn[doc[i] - lo] : (L.fieldnorm ? (uint32_t)__ldg(L.fieldnorm + doc[i]) : 1u);
+          sc[i] = bm25_score_id(scr, id, tf[i]);
+        }
+      }
+    }
+#pragma unroll
+    for (int i = 0; i < 4; ++i)
+      if (doc[i] >= lo && doc[i] < hi) f(doc[i] - lo, sc[i]);
+  }
+}
+
+__global__ void __launch_bounds__(kThreads, 2) k_bool(const BatchParams P, uint32_t unit_base) {
+  extern __shared__ __align__(16) float s_tot[];                          // [kBoolDocs] sum of the group scores
+  float* s_part = s_tot + kBoolDocs;                                      // [kBoolDocs] the current group's score, then the SHOULD sum
+  uint32_t* s_mask = reinterpret_cast<uint32_t*>(s_part + kBoolDocs);     // [kBoolWords] docs still matching
+  uint32_t* s_pres = s_mask + kBoolWords;                                 // [kBoolWords] docs the current group lists
+  uint8_t* s_cnt = reinterpret_cast<uint8_t*>(s_pres + kBoolWords);       // [kBoolDocs] SHOULD clauses listing the doc
+  uint8_t* s_fn = s_cnt + kBoolDocs;                                      // [kBoolDocs] fieldnorm ids of the window
+  __shared__ CtaTopK s_top;
+  __shared__ BoolShared sh;
+  const Unit U = P.units[unit_base + blockIdx.x];
+  const QSeg S = P.qsegs[U.qseg];
+  const DQuery Q = P.queries[S.query];
+  QState* qs = P.qstate + S.query;
+  const uint32_t lane = threadIdx.x & 31u, warp = threadIdx.x >> 5;
+  const float neg_zero = __uint_as_float(0x80000000u);  // -0.0 + s == s bit for bit: a slot holding it takes its first score as is
+  const bool staged_fn = (S.flags & 1u) && S.fieldnorm != nullptr;
+  const bool prunable = (S.flags & 2u) != 0;
+  const uint32_t ng = (S.flags >> 8) & 255u, need = (S.flags >> 16) & 255u;
+  if (threadIdx.x < 32) sh.cur[threadIdx.x] = 0;
+  if (threadIdx.x == 0) {
+    s_top.count = 0; s_top.theta = (unsigned long long)qs->theta << 32;
+    sh.npass = 0;
+    // a doc scores less than the sum of the MUST and SHOULD weights: a clause adds less than its weight (tf/(tf+norm) < 1,
+    // bm25.rs:170-175); used only when every weight is finite and >= 0
+    float sum = 0.0f;
+    for (uint32_t t = 0; t < S.n_lists; ++t) {
+      const QList ql = P.qlists[S.lists_base + t];
+      if ((ql.pad & 3u) != kBoolNot) sum += ql.weight;
+    }
+    sh.bound = sum * 1.00001f;  // f32 sums of up to 32 non-negative terms differ by < 4e-6 relative, whatever the order
+  }
+  __syncthreads();
+  const TopK T{s_top.keys, &s_top.count, &s_top.theta, &s_top.scratch, (unsigned)kThreads};
+  for (uint32_t win = U.begin; win < U.end; ++win) {
+    const uint32_t lo = win * kBoolDocs;
+    const uint32_t hi = min(lo + kBoolDocs, S.max_doc);
+    // ---- block ranges of every clause in this window ---------------------------------------------------------------
+    for (uint32_t t = warp; t < S.n_lists; t += kWarps) {
+      const QList ql = P.qlists[S.lists_base + t];
+      const uint32_t* last_doc = P.lists[ql.list_id].last_doc;
+      const uint32_t n_total = P.lists[ql.list_id].n_total;
+      uint32_t blo = 1, bhi = 0;
+      const uint32_t j_lo = first_block_ge(last_doc, sh.cur[t], n_total, lo, lane);
+      if (j_lo < n_total) {
+        uint32_t j_hi = first_block_ge(last_doc, j_lo, n_total, hi - 1u, lane);  // the last block that can hold a doc < hi
+        if (j_hi >= n_total) j_hi = n_total - 1u;
+        blo = j_lo; bhi = j_hi;
+      }
+      if (lane == 0) { sh.blo[t] = blo; sh.bhi[t] = bhi; sh.cur[t] = j_lo; }
+    }
+    __syncthreads();
+    // ---- skip: a MUST group without a block here, too few SHOULD clauses with one, or a bound under the threshold ------
+    if (threadIdx.x == 0) {
+      const unsigned long long g = (unsigned long long)(*(volatile unsigned int*)&qs->theta) << 32;
+      if (g > s_top.theta) s_top.theta = g;
+      bool skip = prunable && sh.bound < threshold_score((uint32_t)(s_top.theta >> 32));
+      uint32_t n_should = 0, group = 0, group_any = 0;
+      for (uint32_t t = 0; t < S.n_lists && !skip; ++t) {
+        const uint32_t pad = P.qlists[S.lists_base + t].pad;
+        const bool has = sh.blo[t] <= sh.bhi[t];
+        if ((pad & 3u) == kBoolMust) {
+          if ((pad >> 2) != group) { skip = !group_any; group = pad >> 2; group_any = 0; }
+          group_any |= has;
+        } else if ((pad & 3u) == kBoolShould) {
+          n_should += has;
+        }
+      }
+      if (ng && !group_any) skip = true;  // the last group
+      sh.skip = skip || n_should < need;
+    }
+    __syncthreads();
+    if (sh.skip) continue;  // (uniform: read between two barriers; the next write is behind the next window's barrier)
+
+    if (staged_fn) {
+      const uint4* src = reinterpret_cast<const uint4*>(S.fieldnorm + lo);
+      uint4* dst = reinterpret_cast<uint4*>(s_fn);
+      for (uint32_t i = threadIdx.x; i < kBoolDocs / 16; i += kThreads) dst[i] = __ldg(src + i);
+    }
+    for (uint32_t i = threadIdx.x; i < kBoolDocs; i += kThreads) s_part[i] = neg_zero;
+    for (uint32_t w = threadIdx.x; w < kBoolWords; w += kThreads) {
+      const uint32_t first = lo + w * 32u;
+      s_mask[w] = first >= hi ? 0u : (hi - first >= 32u ? 0xFFFFFFFFu : (1u << (hi - first)) - 1u);  // docs below max_doc
+      s_pres[w] = 0;
+    }
+    __syncthreads();
+    // ---- MUST groups ------------------------------------------------------------------------------------------------
+    uint32_t t = 0;
+    bool matching = true;
+    for (uint32_t g = 0; g < ng && matching; ++g) {
+      for (; t < S.n_lists; ++t) {
+        const QList ql = P.qlists[S.lists_base + t];
+        if ((ql.pad & 3u) != kBoolMust || (ql.pad >> 2) != g) break;
+        bool_for_each_posting<true>(P, ql, sh.blo[t], sh.bhi[t], lo, hi, s_fn, staged_fn, warp, lane, [&](uint32_t slot, float sc) {
+          s_part[slot] = __fadd_rn(s_part[slot], sc);
+          atomicOr(&s_pres[slot >> 5], 1u << (slot & 31u));
+        });
+        __syncthreads();  // clause order is the f32 summation order
+      }
+      for (uint32_t i = threadIdx.x; i < kBoolDocs; i += kThreads) {
+        const float v = s_part[i];
+        s_tot[i] = g ? __fadd_rn(s_tot[i], v) : v;
+        s_part[i] = neg_zero;
+      }
+      uint32_t any = 0;
+      for (uint32_t w = threadIdx.x; w < kBoolWords; w += kThreads) {
+        const uint32_t m = s_mask[w] & s_pres[w];
+        s_mask[w] = m;
+        s_pres[w] = 0;
+        any |= m;
+      }
+      matching = __syncthreads_or(any != 0) != 0;
+    }
+    if (!matching) continue;  // no doc of the window has every MUST group
+    // ---- SHOULD clauses: their sum (s_part) and how many list the doc ------------------------------------------------
+    const uint32_t should_begin = t;
+    for (; t < S.n_lists && (P.qlists[S.lists_base + t].pad & 3u) == kBoolShould; ++t) {
+      if (t == should_begin) {
+        for (uint32_t i = threadIdx.x; i < kBoolDocs / 16; i += kThreads) reinterpret_cast<uint4*>(s_cnt)[i] = make_uint4(0, 0, 0, 0);
+        __syncthreads();
+      }
+      bool_for_each_posting<true>(P, P.qlists[S.lists_base + t], sh.blo[t], sh.bhi[t], lo, hi, s_fn, staged_fn, warp, lane, [&](uint32_t slot, float sc) {
+        s_part[slot] = __fadd_rn(s_part[slot], sc);
+        s_cnt[slot] = (uint8_t)(s_cnt[slot] + 1u);  // one posting per doc and clause: no other thread writes this byte now
+      });
+      __syncthreads();
+    }
+    const bool has_should = t > should_begin;
+    // ---- MUST_NOT clauses ---------------------------------------------------------------------------------------------
+    for (; t < S.n_lists; ++t)
+      bool_for_each_posting<false>(P, P.qlists[S.lists_base + t], sh.blo[t], sh.bhi[t], lo, hi, s_fn, staged_fn, warp, lane, [&](uint32_t slot, float) {
+        atomicAnd(&s_mask[slot >> 5], ~(1u << (slot & 31u)));
+      });
+    __syncthreads();
+
+    // ---- harvest: final scores, the float pre-filter, the exact key test on the survivors (as k_or) ------------------
+    const unsigned long long theta = *T.theta;
+    const float theta_f = threshold_score((uint32_t)(theta >> 32));
+    uint32_t passmask = 0;
+#pragma unroll 1
+    for (int j = 0; j < (int)(kBoolDocs / (kThreads * 4)); ++j) {
+      const uint32_t idx = (j * kThreads + threadIdx.x) * 4;
+      const uint32_t bits = (s_mask[idx >> 5] >> (idx & 31u)) & 15u;
+      if (bits) {
+        const float4 tv = *reinterpret_cast<const float4*>(s_tot + idx);
+        const float4 sv = *reinterpret_cast<const float4*>(s_part + idx);
+        const uint32_t cnt4 = has_should ? *reinterpret_cast<const uint32_t*>(s_cnt + idx) : 0u;
+        const float tt[4] = {tv.x, tv.y, tv.z, tv.w}, ss[4] = {sv.x, sv.y, sv.z, sv.w};
+        float vv[4];
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const uint32_t cnt = (cnt4 >> (8 * c)) & 255u;
+          vv[c] = ng ? (cnt ? __fadd_rn(tt[c], ss[c]) : tt[c]) : ss[c];
+          const uint32_t d = lo + idx + c;
+          bool pass = ((bits >> c) & 1u) && cnt >= need && vv[c] >= theta_f && make_key(vv[c], d) >= theta;
+          if (pass && S.alive) pass = is_alive(S.alive, d);
+          passmask |= pass ? (1u << (j * 4 + c)) : 0u;
+        }
+        *reinterpret_cast<float4*>(s_tot + idx) = make_float4(vv[0], vv[1], vv[2], vv[3]);  // read back by the push below
+      }
+    }
+    const uint32_t wsum = __reduce_add_sync(kFull, (uint32_t)__popc(passmask));
+    if (lane == 0 && wsum) atomicAdd(&sh.npass, wsum);
+    __syncthreads();
+    const uint32_t npass = sh.npass;
+    const bool fits = *T.count + npass <= kCap;
+    __syncthreads();
+    if (threadIdx.x == 0) sh.npass = 0;
+    if (!fits) topk_round_end(T, Q.k, &qs->theta);  // cold start: more survivors than the buffer holds; rounds with compaction between
+#pragma unroll 1
+    for (int j = 0; j < (int)(kBoolDocs / (kThreads * 4)); ++j) {
+      const uint32_t idx = (j * kThreads + threadIdx.x) * 4;
+      const uint32_t sub = (passmask >> (j * 4)) & 15u;
+      if (__ballot_sync(kFull, sub != 0)) {
+        const float4 v = *reinterpret_cast<const float4*>(s_tot + idx);
+        const float vv[4] = {v.x, v.y, v.z, v.w};
+        const unsigned long long th = fits ? 0ull : *T.theta;
+#pragma unroll
+        for (int c = 0; c < 4; ++c) {
+          const unsigned long long key = make_key(vv[c], lo + idx + c);
+          topk_push(T, ((sub >> c) & 1u) && key >= th, key, lane);
+        }
+      }
+      if (!fits) topk_round_end(T, Q.k, &qs->theta);
+    }
+    if (fits) topk_round_end(T, Q.k, &qs->theta);
+  }
+  topk_flush(T, Q, qs, P.cands, S.segment_ord);
 }
 
 // The exact k-th largest score key among a query's candidates so far (4-pass radix select) becomes a lower bound of
